@@ -48,6 +48,7 @@ UNIT = "atoms/s"
 FLOP_PAIR = 2 * 32 * 32 + 3 * 32           # per ordered (i,j) pair per GNN step (SURVEY.md 8d): 2144
 FLOP_PAIR_E = 2 * 48 * 32                  # extra for pairs with e != 0: 3072
 FLOP_EPN_PAIR = 2 * (48 * 32 + 2 * (32 * 32 + 32)) + 2 * 64   # per unordered near pair per pass: 7424
+DUMP_MAX_ATOMS = 4_000_000                 # --dump-outputs: 12 B per atom (float32 + float64 charge), at most 48 MB
 
 
 def parse_args():
@@ -78,6 +79,9 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--seed", type=int, default=0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write rank 0's charges of the last timed step to DIR/charges.npy (float32) and "
+                         f"DIR/charges_f64.npy (float64); above {DUMP_MAX_ATOMS} atoms both hold the same fixed, seeded sample of atoms")
     args = ap.parse_args()
     if args.checkpoint is None:
         args.checkpoint = {"qm9_test": "model_weights", "ssi": "model2_weights"}.get(args.workload, "decay_model_weights")
@@ -449,6 +453,18 @@ def conservation(q64, offs, Q):
             "from": "FP64 copy of the charges (q_out_f64); the float32 output rounds each charge by up to 6e-8 |q| on top"}
 
 
+def dump_outputs(out_dir, q32, q64):
+    """--dump-outputs: the charges the device arm's caller holds after the last timed step (q_out float32, q_out64 float64).
+    Above DUMP_MAX_ATOMS atoms both files hold the same atoms, drawn with a fixed seed and kept in atom order, so two builds
+    run with the same arguments can be compared entry for entry."""
+    os.makedirs(out_dir, exist_ok=True)
+    if len(q32) > DUMP_MAX_ATOMS:
+        idx = np.sort(np.random.default_rng(0).choice(len(q32), DUMP_MAX_ATOMS, replace=False))
+        q32, q64 = q32[idx], q64[idx]
+    np.save(os.path.join(out_dir, "charges.npy"), np.ascontiguousarray(q32, np.float32))
+    np.save(os.path.join(out_dir, "charges_f64.npy"), np.ascontiguousarray(q64, np.float64))
+
+
 def secondary_blocks(box, args, main_res, main_value):
     """Driver-visible evidence beyond the headline line (VERDICT r01 items 3 and 8): strong scaling of both multi-GPU configs,
     a live-GNN checkpoint on the headline workload, and the reference's own three configurations.  Short runs (3 steps)."""
@@ -558,6 +574,8 @@ def run_b200(args):
         eng.set_shard(rank, world)
     res = time_case(box, eng, offs, xyz, sp, Q, npad, args.steps, args.warmup, host_too=not args.no_e2e, clocks=True)
     ms_dev, acc, clocks = res["ms_dev"], res["acc"], res["clocks"]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res["q32"], res["q64"])
     e2e = None
     if res["e2e_ms"] is not None:
         e2e = {"value": (1 if sharded_system else world) * n_atoms * args.steps / (res["e2e_ms"] * 1e-3), "unit": UNIT,

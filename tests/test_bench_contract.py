@@ -6,6 +6,8 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -50,12 +52,33 @@ def test_b200_arm_has_no_cpu_fallback():
 import pytest
 
 
+def test_dump_outputs_writes_float_arrays_and_a_fixed_sample(tmp_path, monkeypatch):
+    """--dump-outputs: small outputs are written whole; above the size limit both arrays hold the same seeded sample of atoms
+    in atom order, the same on every run."""
+    sys.path.insert(0, ROOT)
+    import bench
+    q64 = np.arange(5000) + 0.25                     # each value names its atom
+    q32 = (q64 - 0.5).astype(np.float32)
+    bench.dump_outputs(str(tmp_path / "whole"), q32, q64)
+    assert np.array_equal(np.load(tmp_path / "whole" / "charges.npy"), q32)
+    assert np.array_equal(np.load(tmp_path / "whole" / "charges_f64.npy"), q64)
+    monkeypatch.setattr(bench, "DUMP_MAX_ATOMS", 1000)
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), q32, q64)
+    a32, a64 = np.load(tmp_path / "a" / "charges.npy"), np.load(tmp_path / "a" / "charges_f64.npy")
+    assert a32.dtype == np.float32 and a64.dtype == np.float64 and a32.shape == a64.shape == (1000,)
+    atoms = (a64 - 0.25).astype(np.int64)
+    assert np.all(np.diff(atoms) > 0) and np.array_equal(a32, q32[atoms])
+    assert np.array_equal(np.load(tmp_path / "b" / "charges.npy"), a32) and np.array_equal(np.load(tmp_path / "b" / "charges_f64.npy"), a64)
+
+
 @pytest.mark.gpu
-def test_b200_arm_prints_the_contract_line_with_roofline_baseline_and_secondary_blocks():
-    """The driver's own invocation shape (`python bench.py`), shrunk: one JSON line on stdout carrying the base contract, the
+def test_b200_arm_prints_the_contract_line_with_roofline_baseline_and_secondary_blocks(tmp_path):
+    """The default invocation (`python bench.py`), shrunk: one JSON line on stdout carrying the base contract, the
     roofline / cpu_baseline / e2e objects of this tier and the secondary blocks (strong scaling, live-GNN checkpoints, the
-    reference's three own configurations)."""
-    out = _run("--molecules", "20000", "--steps", "2", "--warmup", "3", "--ref-molecules", "64", "--strong-atoms", "3000")
+    reference's three own configurations); --dump-outputs leaves the charges of the last timed step."""
+    out = _run("--molecules", "20000", "--steps", "2", "--warmup", "3", "--ref-molecules", "64", "--strong-atoms", "3000",
+               "--dump-outputs", str(tmp_path))
     assert out.returncode == 0, out.stderr[-800:]
     lines = [ln for ln in out.stdout.splitlines() if ln.strip()]
     assert len(lines) == 1
@@ -77,3 +100,6 @@ def test_b200_arm_prints_the_contract_line_with_roofline_baseline_and_secondary_
     assert s["config_qm9_test"]["precision_used"] == 64 and s["config_ssi"]["precision_used"] == 32
     assert s["config_galectin3c"]["max_abs_dq_vs_reference_preds_npy"] < 1e-5
     assert s["strong_protein"]["checks"]["max_abs_sum_q_minus_Q"] < 1e-6
+    q32, q64 = np.load(tmp_path / "charges.npy"), np.load(tmp_path / "charges_f64.npy")
+    assert q32.dtype == np.float32 and q64.dtype == np.float64 and q32.shape == q64.shape == (d["config"]["atoms_per_gpu_per_step"],)
+    assert np.abs(q32 - q64).max() < 1e-6 and abs(q64.sum()) < 20000 * 1e-6          # 20000 neutral molecules
