@@ -782,9 +782,12 @@ static int probe_precision(epnn_ctx* c, int64_t n_sys, const int32_t* off, bool 
                            const float* Q, const int32_t* npad_host) {
     int64_t ns = n_sys < 64 ? n_sys : 64;
     while (ns > 1 && off[ns] > 8192) --ns;
+    // a first system of more than 8192 atoms: the probe runs on a contiguous cut of its first 8192 atoms, taken as a system
+    // of its own (same Q and npad), so that the choice still rests on the caller's data
+    const int32_t cut_off[2] = {0, 8192};
+    if (off[ns] > 8192) off = cut_off;
     const int64_t na = off[ns];
     c->probe_err32 = c->probe_err48 = -1;
-    if (na > 8192) { c->auto_choice = 32; return EPNN_OK; }       // one big system: three extra inferences would not be a probe
     std::vector<float> hx, hQ, tmp((size_t)na);
     std::vector<int32_t> hs;
     const float* px = xyz; const int32_t* ps = species; const float* pq = Q;

@@ -1,6 +1,8 @@
-// EXPERIMENTAL FP32 kernel for the FAR (e == 0) part of the big-system message sum (option "pair_const" = 1 without
-// "gnn_far_tensor"; precision 32 only; default OFF).  Like the other kernels of that option it has NOT run on a GPU yet;
-// its logic is checked by the CPU warp emulation inside whole inferences (tests/test_emu_infer.py).
+// FP32 kernel for the FAR (e == 0) part of the big-system message sum: the default far kernel of precision 32 for
+// systems of 49 .. 16 383 atoms ("pair_const" 1 or 2, the default 2, whenever the tcgen05 kernel of epnn_gnn_tc.cu is
+// not selected; that one takes over from "gnn_far_tensor_min" = 16 384 atoms).  Checked on the GPU against the float64
+// oracle (tests/test_gpu_large_reference.py, tests/test_gpu_pair_const.py) and by the CPU warp emulation inside whole
+// inferences (tests/test_emu_infer.py).
 //
 // For a row i of a big system the reference sums  m_ij = relu(W2^T relu(u_i + v_j) + b2)  over ALL columns j that are not
 // within the cutoff (charge_gn.py:66-70, no mask) -- the O(n^2) part of a step whenever the far-column de-duplication
