@@ -792,11 +792,14 @@ static int probe_precision(epnn_ctx* c, int64_t n_sys, const int32_t* off, bool 
     std::vector<int32_t> hs;
     const float* px = xyz; const int32_t* ps = species; const float* pq = Q;
     if (!host_io) {
+        // the caller's inputs are ordered on the ctx stream (a caller stream after epnn_set_stream, typically non-blocking):
+        // copy them there, not on the legacy default stream, which would not wait for the kernels that produce them
         hx.resize(3 * (size_t)na); hs.resize((size_t)na); hQ.resize((size_t)ns);
         CU(c, cudaSetDevice(c->device));
-        CU(c, cudaMemcpy(hx.data(), xyz, sizeof(float) * 3 * (size_t)na, cudaMemcpyDeviceToHost));
-        CU(c, cudaMemcpy(hs.data(), species, sizeof(int32_t) * (size_t)na, cudaMemcpyDeviceToHost));
-        CU(c, cudaMemcpy(hQ.data(), Q, sizeof(float) * (size_t)ns, cudaMemcpyDeviceToHost));
+        CU(c, cudaMemcpyAsync(hx.data(), xyz, sizeof(float) * 3 * (size_t)na, cudaMemcpyDeviceToHost, c->stream));
+        CU(c, cudaMemcpyAsync(hs.data(), species, sizeof(int32_t) * (size_t)na, cudaMemcpyDeviceToHost, c->stream));
+        CU(c, cudaMemcpyAsync(hQ.data(), Q, sizeof(float) * (size_t)ns, cudaMemcpyDeviceToHost, c->stream));
+        CU(c, cudaStreamSynchronize(c->stream));
         px = hx.data(); ps = hs.data(); pq = hQ.data();
     }
     // candidates, cheapest first: FP32 with the per-atom kernel on the tensor path (if the option allows it), plain FP32 SIMT,

@@ -1,9 +1,12 @@
 """A WHOLE charge inference on the CPU through the product's own code: weights packed and folded by epnn_pack.h (what
 epnn_create runs), then every kernel of the FP32 path -- neighbour list, descriptors, far lists, bundle kernels, row-group
 kernels, per-atom kernel -- executed by the warp emulation (tools/emu/emu_infer.cpp) in run_chunk's launch order.
-Compared with the float64 oracle and with the reference's own shipped predictions.  Also run with the experimental
-pair-per-thread kernels (epnn_bundle_const.cu, epnn_atom_const.cu), which have not been on a GPU yet, and with the
-mma.sync electron-passing kernel (epnn_bundle_mma.cu; its fragment layout is emulated lane by lane).
+Compared with the float64 oracle and with the reference's own shipped predictions.  Variants ("variant" argument of
+emu_infer): 0 the round-1 warp-tile kernels ("pair_const" 0), 1 the pair-per-thread kernels everywhere (epnn_bundle_const.cu,
+epnn_atom_const.cu, epnn_gnn_far_const.cu; "pair_const" 1), 2 variant 0 with the mma.sync electron-passing kernel
+(epnn_bundle_mma.cu, "pair_tensor" 1; its fragment layout is emulated lane by lane), 3 the shipped FP32 set ("pair_const" 2):
+the row-run GNN bundle kernel (epnn_bundle_run.cu), the pair-per-thread electron-passing bundle kernel and far_const
+for large systems, with the SIMT per-atom kernel (the tensor per-atom kernel has its own emulation test).
 This is test infrastructure, not a fallback: nothing in epnn_b200/ can reach it."""
 import ctypes as C
 import os
@@ -47,7 +50,7 @@ def _infer(emu, w, offs, xyz, sp, Q, npad, pair_const=0, dedup=1):
     return q32, q64, h, int(rows[0])
 
 
-@pytest.mark.parametrize("pair_const", [0, 1, 2])      # 0 default kernels, 1 experimental pair_const, 2 pair_tensor (mma.sync EPN kernel)
+@pytest.mark.parametrize("pair_const", [0, 1, 2, 3])      # the emulated kernel set ("variant", see the module docstring)
 def test_emulated_inference_reproduces_shipped_predictions(emu, weights, mixed, val871, pair_const):
     """decay_model_weights, pad 41: the reference's own predictions (models/model_systems/test_pred_charges.npy)."""
     w = weights["decay_model_weights"]
@@ -64,7 +67,7 @@ def test_emulated_inference_reproduces_shipped_predictions(emu, weights, mixed, 
 
 
 @pytest.mark.parametrize("name", ["model2_weights", "model_weights"])
-@pytest.mark.parametrize("pair_const", [0, 1, 2])
+@pytest.mark.parametrize("pair_const", [0, 1, 2, 3])
 def test_emulated_inference_live_checkpoints(emu, weights, mixed, name, pair_const):
     """Checkpoints whose hidden state is live: charges AND the GNN-layer output against the oracle (only step 0 collapses)."""
     w = weights[name]
@@ -82,7 +85,7 @@ def test_emulated_inference_live_checkpoints(emu, weights, mixed, name, pair_con
         assert np.abs(h[offs[k]:offs[k + 1]] - tr["h"]).max() < 2e-4 * np.abs(tr["h"]).max(), (name, k)
 
 
-@pytest.mark.parametrize("pair_const,dedup", [(0, 1), (0, 0), (1, 1)])
+@pytest.mark.parametrize("pair_const,dedup", [(0, 1), (0, 0), (1, 1), (3, 1), (3, 0)])
 def test_emulated_inference_with_a_large_system(emu, weights, mixed, protein, pair_const, dedup):
     """A 90-atom protein cut (row-group kernels, three partial-sum planes, species tables) between two small molecules."""
     w = weights["decay_model_weights"]
@@ -101,7 +104,7 @@ def test_emulated_inference_with_a_large_system(emu, weights, mixed, protein, pa
     assert rows == (3 * 90 if dedup else 0)                              # 3 of the 5 steps collapse for this checkpoint (DESIGN.md)
 
 
-@pytest.mark.parametrize("seed,pair_const", [(1, 0), (2, 0), (3, 1)])
+@pytest.mark.parametrize("seed,pair_const", [(1, 0), (2, 0), (3, 1), (4, 3)])
 def test_emulated_inference_random_systems(emu, weights, seed, pair_const):
     """Randomly sized synthetic systems (1 .. 48 atoms and a few larger ones, jittered-lattice geometries, random species
     and net charges, padded and unpadded) -- tile and bundle boundaries fall wherever they fall."""

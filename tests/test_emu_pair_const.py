@@ -1,4 +1,5 @@
-"""CPU warp emulation of the (GPU-unvalidated) pair-per-thread bundle kernels, epnn_b200/csrc/epnn_bundle_const.cu.
+"""CPU warp emulation of the pair-per-thread bundle kernels, epnn_b200/csrc/epnn_bundle_const.cu ("pair_const" 1; its
+electron-passing variant is also part of the FP32 default set, "pair_const" 2).
 
 The kernel source is compiled for the host with -DEPNN_CPU_EMU (tools/emu/cuda_emu.h: every lane is a host thread,
 shuffles / votes / __syncwarp through a per-warp barrier, shared memory a host buffer) and run on index lists built here
@@ -6,7 +7,7 @@ from the reference's own molecules exactly the way the CUDA prep kernels build t
 far lists, species-compressed far lists, representatives).  Its outputs -- the message sums S of a message-passing step
 and the per-pair transfers delta of an electron-passing pass -- are compared with a direct float64 evaluation of the
 reference formulas (charge_gn.py:62-70, :101-116).  This checks the kernel's indexing, control flow, shared-memory
-layout and summation logic before it ever reaches a GPU; it says nothing about performance."""
+layout and summation logic without a GPU; it says nothing about performance."""
 import ctypes as C
 import os
 import subprocess

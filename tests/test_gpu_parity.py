@@ -360,6 +360,47 @@ def test_caller_stream_and_device_pointers(weights, mixed):
         eng.close()
 
 
+def test_caller_stream_precision_probe_reads_the_callers_inputs(weights, mixed):
+    """"precision" 0 with device pointers on a caller stream: the precision probe reads its prefix of the inputs on that
+    stream, after the kernels that write them.  The input buffers hold zeros until a copy that the caller stream runs
+    after a ~100 ms sleep, without a host sync: a probe ordered on any other stream would choose from the zeros (and
+    the choice is sticky).  Same precision, same probe error and the same charges as a host-buffer call."""
+    import torch
+    from epnn_b200.engine import Engine
+    w = weights["model_weights"]
+    idx = mixed.usable(w.n_x)[:600:3].tolist()
+    offs, xyz, sp, Q = mixed.batch(idx, w.n_x)
+    npad = np.full(len(idx), 41, np.int32)
+    n = int(offs[-1])
+    host = Engine(w, device=0, precision=0)
+    try:
+        ref32, ref64 = host.infer_batch(offs, xyz, sp, Q, npad, want_f64=True)
+        ref_st = host.last_stats
+    finally:
+        host.close()
+    eng = Engine(w, device=0, precision=0)
+    try:
+        src = [torch.from_numpy(a).cuda() for a in (xyz, sp, Q)]
+        dst = [torch.zeros_like(a) for a in src]
+        d_out, d_out64 = torch.empty(n, dtype=torch.float32, device="cuda"), torch.empty(n, dtype=torch.float64, device="cuda")
+        torch.cuda.synchronize()
+        st = torch.cuda.Stream()
+        eng.set_stream(st.cuda_stream)
+        with torch.cuda.stream(st):
+            torch.cuda._sleep(200_000_000)                             # about 100 ms at B200 clocks
+            for d, s in zip(dst, src):
+                d.copy_(s)
+            eng.infer_batch_dev(offs, dst[0].data_ptr(), dst[1].data_ptr(), dst[2].data_ptr(), npad, d_out.data_ptr(), d_out64.data_ptr())
+        got = eng.last_stats
+        st.synchronize()
+        eng.set_stream(0)
+    finally:
+        eng.close()
+    assert got["precision_used"] == ref_st["precision_used"] == 64
+    assert got["probe_err32"] == ref_st["probe_err32"] and got["probe_err48"] == ref_st["probe_err48"]
+    assert np.array_equal(d_out.cpu().numpy(), ref32) and np.array_equal(d_out64.cpu().numpy(), ref64)
+
+
 def test_edge_cases(engines, weights):
     w = weights["decay_model_weights"]
     eng = engines("decay_model_weights", 64)
@@ -452,11 +493,8 @@ def test_big_system_charges_and_chunk_of_mixed_sizes(engines, weights, protein, 
     assert np.abs(q[offs[-1]:offs[-1] + n] - protein["preds"]).max() < TOL
 
 
-def test_bundle_boundaries_and_routing(engines, weights, protein):
-    """Sizes around the bundle capacity (48) and the small/large routing threshold, many 1-atom systems, systems
-    that exactly fill a bundle, pad sizes equal to / far above n -- all in one batch, FP64 kernels vs the oracle."""
-    w = weights["model2_weights"]
-    eng = engines("model2_weights", 64)
+def boundary_batch(protein):
+    """Cuts of the protein at sizes around the bundle capacity (48) and the small/large routing threshold."""
     sizes = [1, 1, 1, 47, 1, 48, 49, 50, 24, 24, 24, 25, 23, 1, 48, 2, 46, 3]
     pz = O.species_from_Z(protein["Z"], 9)
     offs = [0]
@@ -474,13 +512,22 @@ def test_bundle_boundaries_and_routing(engines, weights, protein):
     sp = np.concatenate(sp).astype(np.int32)
     Q = np.array(Q, np.float32)
     npad = np.array(npad, np.int32)
+    return offs, xyz, sp, Q, npad
+
+
+def test_bundle_boundaries_and_routing(engines, weights, protein):
+    """Sizes around the bundle capacity (48) and the small/large routing threshold, many 1-atom systems, systems
+    that exactly fill a bundle, pad sizes equal to / far above n -- all in one batch, FP64 kernels vs the oracle."""
+    w = weights["model2_weights"]
+    eng = engines("model2_weights", 64)
+    offs, xyz, sp, Q, npad = boundary_batch(protein)
     q, q64 = eng.infer_batch(offs, xyz, sp, Q, npad, want_f64=True)
     ref = O.predict_batch(w, offs, xyz, sp, Q, npad)
     assert np.abs(q64 - ref).max() < 1e-8 * max(1.0, np.abs(ref).max())
     assert eng.last_stats["n_row_groups"] > 0
-    # the FP32 default path on the same batch
+    # the FP32 default path on the same batch: measured 7.6e-7 on a B200 (1 000 W; tools/measure_small_floor.py), bound 3x
     q32 = engines("model2_weights").infer_batch(offs, xyz, sp, Q, npad, want_f64=True)[1]
-    assert np.abs(q32 - ref).max() < 5e-5 * max(1.0, np.abs(ref).max())
+    assert np.abs(q32 - ref).max() < 2.3e-6 * max(1.0, np.abs(ref).max())
 
 
 def test_synthetic_qm9_stream_properties(engines, weights):

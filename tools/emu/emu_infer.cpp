@@ -2,7 +2,9 @@
 //
 // Weights are packed / folded by the product's own host code (epnn_pack.h, the code epnn_create runs); then the kernels
 // of epnn_neighbor / epnn_bundle / epnn_gnn / epnn_epn / epnn_atom (and, with variant = 1, epnn_bundle_const /
-// epnn_atom_const; with variant = 2, the mma.sync electron-passing kernel epnn_bundle_mma) run in the launch order of
+// epnn_atom_const; with variant = 2, the mma.sync electron-passing kernel epnn_bundle_mma; with variant = 3, the shipped
+// FP32 set of "pair_const" 2: the row-run GNN bundle kernel epnn_bundle_run, the electron-passing kernel of
+// epnn_bundle_const and the far_const kernel for large systems, with the SIMT per-atom kernel) run in the launch order of
 // run_chunk (epnn_api.cu), FP32, one chunk.  The only code that is not the product's is this orchestration (a
 // restatement of run_chunk without streams and workspaces) and two host-side scans.
 // tests/test_emu_infer.py compares the result with the oracle and with the reference's shipped predictions.
@@ -37,6 +39,9 @@ namespace k_farc {
 namespace k_mma {
 #include "../../epnn_b200/csrc/epnn_bundle_mma.cu"
 }
+namespace k_brun {
+#include "../../epnn_b200/csrc/epnn_bundle_run.cu"
+}
 
 static void exclusive_scan(const int* in, int* out, int n) { int s = 0; for (int i = 0; i < n; ++i) { out[i] = s; s += in[i]; } out[n] = s; }
 
@@ -44,7 +49,7 @@ extern "C" int emu_infer(int T, int n_x, const float* w_packed, size_t n_w, int 
                          const int* species, const float* Q, const int* npad_in, int variant, int dedup,
                          float* q_out, double* q_out64, float* h_out, long long* dedup_rows_out) {
     if (n_w != expected_floats(T, n_x)) return -1;
-    const int pair_const = variant == 1, pair_tensor = variant == 2;
+    const int pair_const = variant == 1, pair_tensor = variant == 2, run_set = variant == 3;
     const int n = off[n_sys];
     const int n_species = n_x - 1;
     // ---------------------------------------------------------------- weights: the product's own packing and folding
@@ -137,6 +142,9 @@ extern "C" int emu_infer(int T, int n_x, const float* w_packed, size_t n_w, int 
         emu_launch_simple(div_up(n, 128), 128, [&] {
             k_bundle::far0_kernel<1>(n, atom_sys.data(), off, npad.data(), species, rowptr.data(), col.data(), atom_b0.data(), nullptr, nullptr,
                                      far0_off.data(), far0_list.data(), far0_w.data()); });
+    std::vector<unsigned char> rowl(nnz + 16, 0);
+    if (run_set && n_bundles && nnz > 0)
+        emu_launch_simple(div_up(n, 256), 256, [&] { k_brun::csr_rowl_kernel(n, atom_sys.data(), off, rowptr.data(), atom_b0.data(), rowl.data()); });
     std::vector<int> rgl_off(n_sys + 1, 0), rg;
     for (int s = 0; s < n_sys; ++s) {
         const int ns = off[s + 1] - off[s];
@@ -204,7 +212,21 @@ extern "C" int emu_infer(int T, int n_x, const float* w_packed, size_t n_w, int 
             emu_launch_cta(MMA_NW, (size_t)MMA_NW * BUNDLE_ATOMS * UVS, [&] { k_mma::bundle_epn_mma_kernel(a); });
             return;
         }
-        if (pair_const) {
+        if (run_set && !epn) {
+            k_brun::RunW W;
+            memcpy(W.W2, sw.W2, sizeof(W.W2));
+            k_brun::RunArgs a;
+            memset(&a, 0, sizeof(a));
+            a.n_bundles = n_bundles; a.bundle = bundles.data(); a.work_counter = &work_counter;
+            a.rowptr = rowptr.data(); a.col = col.data(); a.pid = pid.data(); a.rowl = rowl.data(); a.e = e.data(); a.ustart = ustart.data();
+            a.far_off = far_off.data(); a.far_list = far_list.data();
+            a.far0_off = far0_off.data(); a.far0_list = far0_list.data(); a.far0_w = far0_w.data(); a.rep = rep.data(); a.dedup = dedup;
+            a.atom_sys = atom_sys.data(); a.sys_off = off; a.npad = npad.data(); a.u = u.data(); a.v = v.data(); a.S = S.data();
+            a.Cw = sw.Cw; a.b2 = sw.b2; a.b1 = sw.b1;
+            emu_launch_cta(RUN_NW, k_brun::RunSmem::bytes() / sizeof(float), [&] { k_brun::bundle_run_kernel(W, &a); });
+            return;
+        }
+        if (pair_const || run_set) {
             k_bconst::PairW W;
             memcpy(W.W2, sw.W2, sizeof(W.W2));
             k_bconst::ConstArgs a;
@@ -240,9 +262,9 @@ extern "C" int emu_infer(int T, int n_x, const float* w_packed, size_t n_w, int 
                     k_gnn::sp_check_kernel<float>(n, atom_sys.data(), off, species, rgl_off.data(), sp_tab.data(), v.data(), sp_stamp.data(), stamp); });
                 emu_launch_simple(div_up(n_sp_tab, 256), 256, [&] { k_gnn::sp_tally_kernel(n_sp_tab, sp_tab.data(), sp_stamp.data(), stamp, &dedup_rows); });
             }
-            // variant 1: the far columns of the live steps go to the row-per-thread kernel (planes 0 .. nsplit - 2), gnn_pair_kernel keeps
-            // the near pairs, the pad pair and the species slots on the last plane -- the far_tc == 2 arrangement of run_chunk
-            const bool far_const = pair_const;
+            // variants 1 and 3: the far columns of the live steps go to the row-per-thread kernel (planes 0 .. nsplit - 2), gnn_pair_kernel
+            // keeps the near pairs, the pad pair and the species slots on the last plane -- the far_tc == 2 arrangement of run_chunk
+            const bool far_const = pair_const || run_set;
             if (far_const) {
                 std::vector<int2> blk;
                 for (int s = 0; s < n_sys; ++s)
