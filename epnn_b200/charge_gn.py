@@ -154,6 +154,10 @@ class Model:
     def predict_packed(self, offsets, xyz, species, Q, npad=None, want_f64: bool = False):
         return self._need().infer_batch(offsets, xyz, species, Q, npad, want_f64=want_f64)
 
+    def electrostatics(self, offsets, xyz, q, fragment=None, potential: bool = False):
+        """Energy, dipole and optionally potential of given charges: :meth:`epnn_b200.engine.Engine.electrostatics`."""
+        return self._need().electrostatics(offsets, xyz, q, fragment=fragment, potential=potential)
+
     def predict_systems(self, systems: Sequence[xyzio.System], npad=None) -> List[np.ndarray]:
         """Charges of parsed systems through the packed path; ``npad`` = pad size N of the reference's dense model
         (default: the largest system, as ``gen_padded_init_state`` pads, charge_gn.py:340)."""

@@ -11,6 +11,7 @@
 #include <string>
 #include <vector>
 
+#include "epnn_elst.cuh"
 #include "epnn_internal.cuh"
 #include "epnn_pack.h"
 
@@ -111,7 +112,8 @@ static thread_local std::string g_create_err;
 enum {
     B_XYZ, B_SPECIES, B_OFF, B_Q, B_NPAD, B_ATOMSYS, B_DEG, B_DEGU, B_ROWPTR, B_USTART, B_COL, B_PID, B_PI, B_PJ, B_PD,
     B_E, B_NEAR, B_BUNDLE, B_RGL, B_FARCNT, B_FAROFF, B_FARLIST, B_FAR0CNT, B_FAR0OFF, B_FAR0LIST, B_FAR0W, B_REP, B_ATOMB0, B_BNAT, B_PERM, B_LARGESYS, B_GRID, B_CELLCNT, B_CELLSTART, B_CELLATOMS, B_DTMP, B_H, B_L2, B_S, B_U, B_V, B_DELTA, B_QD, B_SCANTMP, B_CNTL, B_RGLOFF,
-    B_OUT32, B_OUT64, B_MISC, B_OFFIN, B_SPTAB, B_SPSTAMP, B_ROWBLK, B_ROWL, B_ARGS, B_DEGALL, B_ACTIVE, B_XYZ_1, B_SPECIES_1, B_Q_1, B_OUT32_1, B_OUT64_1, B_OFFIN_1, B_BPMASK, B_BPTOT, B_BPOFF, B_COUNT
+    B_OUT32, B_OUT64, B_MISC, B_OFFIN, B_SPTAB, B_SPSTAMP, B_ROWBLK, B_ROWL, B_ARGS, B_DEGALL, B_ACTIVE, B_XYZ_1, B_SPECIES_1, B_Q_1, B_OUT32_1, B_OUT64_1, B_OFFIN_1, B_BPMASK, B_BPTOT, B_BPOFF,
+    B_EL_OFF, B_EL_XYZ, B_EL_Q, B_EL_FRAG, B_EL_E, B_EL_MU, B_EL_PHI, B_EL_PLAN, B_EL_PART, B_COUNT
 };
 
 static int fail(epnn_ctx* c, int code, const char* fmt, ...) {
@@ -983,6 +985,86 @@ extern "C" int epnn_infer_batch_dev(epnn_ctx* c, int64_t n_sys, const int32_t* o
                                     const int32_t* species_dev, const float* Q_dev, const int32_t* npad_host,
                                     float* q_out_dev, double* q_out64_dev, epnn_stats* stats) {
     return infer_impl(c, n_sys, off_host, false, xyz_dev, species_dev, Q_dev, npad_host, q_out_dev, q_out64_dev, stats);
+}
+
+// ------------------------------------------------------------------------------------------------
+// Electrostatics of given charges (epnn_elst.cu).  Chunks of plan_chunks (whole systems) run one after the other on the ctx
+// stream; the stream orders the reuse of every workspace, so the call synchronises once, at the end.
+static int elst_impl(epnn_ctx* c, int64_t n_sys, const int32_t* off, bool host_io, const float* xyz, const double* q,
+                     const int32_t* frag, double* energy, double* dipole, double* phi) {
+    if (!c) return EPNN_E_INVALID;
+    int rc = validate_offsets(c, n_sys, off);
+    if (rc != EPNN_OK) return rc;
+    if (n_sys == 0) return EPNN_OK;
+    if (!xyz || !q) return fail(c, EPNN_E_INVALID, "NULL input pointer (xyz or q)");
+    if (!energy && !dipole && !phi) return fail(c, EPNN_E_INVALID, "every output pointer is NULL (energy_out, dipole_out, phi_out)");
+    CU(c, cudaSetDevice(c->device));
+    cudaStream_t st = c->stream;
+    std::vector<int64_t> bounds;
+    plan_chunks(off, n_sys, c->chunk_atoms, bounds);
+    std::vector<ElstItem> items;
+    std::vector<ElstSys> sys;
+    void* p;
+    for (size_t ci = 0; ci + 1 < bounds.size(); ++ci) {
+        const int64_t s0 = bounds[ci], s1 = bounds[ci + 1];
+        const int ns = (int)(s1 - s0), a0 = off[s0], na = off[s1] - off[s0];
+        const long long plen = elst_plan(off + s0, ns, (int64_t)c->sm_count * ELST_CTAS_PER_SM, items, sys);
+        ElstArgs a;
+        a.n_sys = ns; a.base = a0;
+        if ((rc = ensure(c, B_EL_OFF, sizeof(int) * ((size_t)ns + 1), &p)) != EPNN_OK) return rc;
+        a.off = (const int*)p;
+        CU(c, cudaMemcpyAsync(p, off + s0, sizeof(int) * ((size_t)ns + 1), cudaMemcpyHostToDevice, st));
+        const size_t items_bytes = sizeof(ElstItem) * items.size(), sys_bytes = sizeof(ElstSys) * sys.size();
+        a.items = nullptr; a.sys = nullptr; a.partial = nullptr;
+        if (!items.empty()) {
+            if ((rc = ensure(c, B_EL_PLAN, items_bytes + sys_bytes, &p)) != EPNN_OK) return rc;
+            CU(c, cudaMemcpyAsync(p, items.data(), items_bytes, cudaMemcpyHostToDevice, st));
+            CU(c, cudaMemcpyAsync((char*)p + items_bytes, sys.data(), sys_bytes, cudaMemcpyHostToDevice, st));
+            a.items = (const ElstItem*)p; a.sys = (const ElstSys*)((char*)p + items_bytes);
+            if ((rc = ensure(c, B_EL_PART, sizeof(double) * (size_t)plen, &p)) != EPNN_OK) return rc;
+            a.partial = (double*)p;
+        }
+        if (host_io) {
+            if ((rc = ensure(c, B_EL_XYZ, sizeof(float) * 3 * (size_t)na, &p)) != EPNN_OK) return rc;
+            a.xyz = (const float*)p;
+            CU(c, cudaMemcpyAsync(p, xyz + 3 * (size_t)a0, sizeof(float) * 3 * (size_t)na, cudaMemcpyHostToDevice, st));
+            if ((rc = ensure(c, B_EL_Q, sizeof(double) * (size_t)na, &p)) != EPNN_OK) return rc;
+            a.q = (const double*)p;
+            CU(c, cudaMemcpyAsync(p, q + a0, sizeof(double) * (size_t)na, cudaMemcpyHostToDevice, st));
+            a.frag = nullptr;
+            if (frag) {
+                if ((rc = ensure(c, B_EL_FRAG, sizeof(int) * (size_t)na, &p)) != EPNN_OK) return rc;
+                a.frag = (const int*)p;
+                CU(c, cudaMemcpyAsync(p, frag + a0, sizeof(int) * (size_t)na, cudaMemcpyHostToDevice, st));
+            }
+            a.energy = a.dipole = a.phi = nullptr;
+            if (energy) { if ((rc = ensure(c, B_EL_E, sizeof(double) * (size_t)ns, &p)) != EPNN_OK) return rc; a.energy = (double*)p; }
+            if (dipole) { if ((rc = ensure(c, B_EL_MU, sizeof(double) * 3 * (size_t)ns, &p)) != EPNN_OK) return rc; a.dipole = (double*)p; }
+            if (phi) { if ((rc = ensure(c, B_EL_PHI, sizeof(double) * (size_t)na, &p)) != EPNN_OK) return rc; a.phi = (double*)p; }
+        } else {
+            a.xyz = xyz + 3 * (size_t)a0; a.q = q + a0; a.frag = frag ? frag + a0 : nullptr;
+            a.energy = energy ? energy + s0 : nullptr; a.dipole = dipole ? dipole + 3 * s0 : nullptr; a.phi = phi ? phi + a0 : nullptr;
+        }
+        CU(c, launch_elst(a, (int)items.size(), (int)sys.size(), st));
+        if (host_io) {
+            if (energy) CU(c, cudaMemcpyAsync(energy + s0, a.energy, sizeof(double) * (size_t)ns, cudaMemcpyDeviceToHost, st));
+            if (dipole) CU(c, cudaMemcpyAsync(dipole + 3 * s0, a.dipole, sizeof(double) * 3 * (size_t)ns, cudaMemcpyDeviceToHost, st));
+            if (phi) CU(c, cudaMemcpyAsync(phi + a0, a.phi, sizeof(double) * (size_t)na, cudaMemcpyDeviceToHost, st));
+        }
+    }
+    CU(c, cudaStreamSynchronize(st));
+    return EPNN_OK;
+}
+
+extern "C" int epnn_electrostatics(epnn_ctx* c, int64_t n_sys, const int32_t* off, const float* xyz, const double* q,
+                                   const int32_t* fragment, double* energy_out, double* dipole_out, double* phi_out) {
+    return elst_impl(c, n_sys, off, true, xyz, q, fragment, energy_out, dipole_out, phi_out);
+}
+
+extern "C" int epnn_electrostatics_dev(epnn_ctx* c, int64_t n_sys, const int32_t* off_host, const float* xyz_dev,
+                                       const double* q_dev, const int32_t* fragment_dev, double* energy_out_dev,
+                                       double* dipole_out_dev, double* phi_out_dev) {
+    return elst_impl(c, n_sys, off_host, false, xyz_dev, q_dev, fragment_dev, energy_out_dev, dipole_out_dev, phi_out_dev);
 }
 
 // ------------------------------------------------------------------------------------------------

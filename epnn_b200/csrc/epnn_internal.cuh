@@ -347,6 +347,8 @@ cudaError_t launch_atom_mixed(const Workspace& w, int mode, const StepW<double>*
 cudaError_t launch_atom_mma(const Workspace& w, const AtomArgs<float, float>& aa, cudaStream_t st, int* n_launch);   // option atom_tensor (epnn_atom_mma.cu)
 cudaError_t launch_atom_const(const Workspace& w, int mode, const StepW<float>* prev, const UpdW<float>* upd, const StepW<float>* next,
                               int h_is_zero, float* q_out, double* q_out64, cudaStream_t st, int* n_launch);   // option pair_const
+struct ElstArgs;
+cudaError_t launch_elst(const ElstArgs& a, int n_items, int n_large, cudaStream_t st);   // epnn_elst.cu (plan: epnn_elst.cuh)
 
 #endif   // !EPNN_CPU_EMU
 static inline int div_up(int64_t a, int64_t b) { return (int)((a + b - 1) / b); }

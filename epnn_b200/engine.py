@@ -10,6 +10,10 @@ import numpy as np
 from . import _capi
 from .checkpoint import Weights
 
+# Unit conversions of the electrostatics outputs (the C-ABI works in e and Angstrom)
+COULOMB_KCAL = 332.0637133       # e^2/A -> kcal/mol: e^2 / (4 pi eps0 A) in kcal/mol, CODATA 2018
+DEBYE_PER_E_ANGSTROM = 4.80320471   # e*A -> Debye, CODATA 2018
+
 
 def _ptr(a: Optional[np.ndarray]):
     return None if a is None else a.ctypes.data_as(C.c_void_p)
@@ -145,6 +149,39 @@ class Engine:
                                                   C.c_void_p(species_dev), C.c_void_p(Q_dev), _ptr(npad_a),
                                                   C.c_void_p(q_out_dev), C.c_void_p(q_out64_dev or None), C.byref(st)))
         self.last_stats = st.as_dict()
+
+    def electrostatics(self, offsets, xyz, q, fragment=None, potential: bool = False):
+        """Coulomb energy (e^2/A), dipole (e*A, about the unweighted centroid) and, with ``potential``, the potential at
+        every atom (e/A) of each system of a packed batch, in FP64 on the GPU (epnn_electrostatics in
+        include/epnn_b200.h).  ``q`` is one charge per atom (float32 charges are widened to float64); ``fragment`` is an
+        optional int label per atom: only pairs with different labels count in the energy and the potential, so a
+        dimer labelled by its split gives the inter-monomer energy.  Returns ``{"energy": (S,), "dipole": (S, 3)
+        [, "phi": (n_atoms,)]}`` float64 arrays."""
+        offsets = _as(offsets, np.int32)
+        xyz = _as(xyz, np.float32)
+        q = _as(q, np.float64)
+        n_sys = offsets.shape[0] - 1
+        n_atoms = int(offsets[-1]) if n_sys >= 0 and offsets.size else 0
+        frag = None if fragment is None else _as(fragment, np.int32)
+        if xyz.size != 3 * n_atoms or q.size != n_atoms or (frag is not None and frag.size != n_atoms):
+            raise ValueError("array sizes are inconsistent with atom_offsets")
+        out = {"energy": np.empty(n_sys, np.float64), "dipole": np.empty((n_sys, 3), np.float64)}
+        if potential:
+            out["phi"] = np.empty(n_atoms, np.float64)
+        self._check(self.lib.epnn_electrostatics(self._h, n_sys, _ptr(offsets), _ptr(xyz), _ptr(q), _ptr(frag),
+                                                 _ptr(out["energy"]), _ptr(out["dipole"]), _ptr(out.get("phi"))))
+        return out
+
+    def electrostatics_dev(self, offsets_host, xyz_dev: int, q_dev: int, fragment_dev: int = 0, energy_dev: int = 0,
+                           dipole_dev: int = 0, phi_dev: int = 0):
+        """Device-pointer variant of :meth:`electrostatics`: the ``*_dev`` arguments are raw CUDA device addresses (ints,
+        0 = NULL); ``q_dev`` holds float64 charges, e.g. the ``q_out64_dev`` of :meth:`infer_batch_dev`."""
+        offsets_host = _as(offsets_host, np.int32)
+        n_sys = offsets_host.shape[0] - 1
+        self._check(self.lib.epnn_electrostatics_dev(self._h, n_sys, _ptr(offsets_host), C.c_void_p(xyz_dev),
+                                                     C.c_void_p(q_dev), C.c_void_p(fragment_dev or None),
+                                                     C.c_void_p(energy_dev or None), C.c_void_p(dipole_dev or None),
+                                                     C.c_void_p(phi_dev or None)))
 
     def neighbors(self, offsets, xyz, which: int = 0):
         """(rowptr, col) CSR of the is_near set (which=0) or the e != 0 set (which=1); global atom indices."""

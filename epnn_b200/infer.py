@@ -26,6 +26,21 @@ def test_step(h, e, x, q, y, mask):
     return model([h, e, x, q, mask])
 
 
+def save_electrostatics(path, model, base, stems, offsets, xyz, q64):
+    """``--elst``: Coulomb energy and dipole of every system, and for the dimers that carry a ``<stem>splits.npy`` the
+    energy between the two monomers and the charge of the first one, from the FP64 charges of the run."""
+    from .engine import COULOMB_KCAL, DEBYE_PER_E_ANGSTROM
+    split = xyzio.read_splits(base, stems)
+    full = model.electrostatics(offsets, xyz, q64)
+    inter = model.electrostatics(offsets, xyz, q64, fragment=xyzio.fragments_from_splits(offsets, split))
+    has = split >= 0
+    q_first = np.full(len(stems), np.nan)
+    q_first[has] = [q64[offsets[i]:offsets[i] + split[i]].sum() for i in np.nonzero(has)[0]]
+    np.savez(path, names=np.array(stems), energy_kcal=full["energy"] * COULOMB_KCAL,
+             inter_kcal=np.where(has, inter["energy"] * COULOMB_KCAL, np.nan), split=split, q_first_fragment=q_first,
+             dipole_debye=full["dipole"] * DEBYE_PER_E_ANGSTROM)
+
+
 def main(argv=None):
     global model
     ap = argparse.ArgumentParser(description=__doc__, formatter_class=argparse.RawDescriptionHelpFormatter)
@@ -40,7 +55,13 @@ def main(argv=None):
     ap.add_argument("--precision", type=int, default=32, choices=[32, 64])
     ap.add_argument("--option", action="append", default=[], metavar="KEY=VALUE",
                     help="engine option (epnn_set_option), e.g. gnn_far_tensor=1, pair_tensor=1, dedup_far=0; repeatable")
+    ap.add_argument("--elst", default=None, metavar="OUT.npz",
+                    help="also save the electrostatics of the predicted FP64 charges (packed path only): names, energy_kcal, "
+                         "inter_kcal and q_first_fragment of the two monomers of each <stem>splits.npy dimer (NaN without "
+                         "one), split, dipole_debye")
     args = ap.parse_args(argv)
+    if args.elst and args.dense:
+        ap.error("--elst needs the packed path (drop --dense)")
     options = []
     for kv in args.option:
         k, sep, v = kv.partition("=")
@@ -88,9 +109,14 @@ def main(argv=None):
         np.save("test_names.npy", names, allow_pickle=True)
         runs = []
         timeC = timeD = time.time()
+        q64 = None
         for _ in range(args.repeats):
             timeC = time.time()
-            runs.append(model.predict_packed(offsets, xyz_all, species_all, Q_all, N))
+            if args.elst:
+                q32, q64 = model.predict_packed(offsets, xyz_all, species_all, Q_all, N, want_f64=True)
+                runs.append(q32)
+            else:
+                runs.append(model.predict_packed(offsets, xyz_all, species_all, Q_all, N))
             timeD = time.time()
             print(timeD - timeC)
         S = len(stems)
@@ -106,6 +132,8 @@ def main(argv=None):
             if os.path.exists(lab):
                 yv = np.array(np.load(lab), dtype=np.float32).reshape(-1)[:sizes[i]]
                 y[i, :len(yv), 0] = yv
+        if args.elst:
+            save_electrostatics(args.elst, model, base, stems, offsets, xyz_all, q64)
 
     print(f"avg inference time: {(timeD - timeC) / max(1, args.repeats)}")
     print(f"avg feature time:{(timeB - timeA)}")

@@ -73,6 +73,45 @@ def pack(systems: Sequence[System], n_x: int):
     return offsets, np.ascontiguousarray(xyz), np.ascontiguousarray(species, dtype=np.int32), Q
 
 
+def read_splits(path: str, stems: Sequence[str]) -> np.ndarray:
+    """For each stem, the index where the second monomer starts, read from ``<path>/<stem>splits.npy`` (the SSI dimers of
+    the reference's data set carry one; ``charge_gn.py:305-308`` loads it), or -1.  A missing file gives -1 silently; a
+    file that does not hold one integer index inside [1, n - 1] of its system gives -1 with a warning (n is read from
+    the atom lines of ``<stem>.xyz``)."""
+    import warnings
+    out = np.full(len(stems), -1, np.int64)
+    for k, stem in enumerate(stems):
+        f = os.path.join(path, stem + "splits.npy")
+        if not os.path.exists(f):
+            continue
+        try:
+            a = np.load(f, allow_pickle=False)
+            n = read_xyz(os.path.join(path, stem + ".xyz")).n
+        except Exception as e:      # noqa: BLE001 -- an unreadable split file is reported, not fatal
+            warnings.warn(f"{f}: cannot be read ({e}); no split")
+            continue
+        v = a.reshape(-1)[0] if a.size == 1 else None
+        if v is None or not (a.dtype.kind in "iu" or (a.dtype.kind == "f" and np.isfinite(v) and float(v).is_integer())):
+            warnings.warn(f"{f}: expected one integer index, got shape {a.shape} dtype {a.dtype}; no split")
+            continue
+        v = int(v)
+        if not 1 <= v <= n - 1:
+            warnings.warn(f"{f}: split {v} is outside [1, {n - 1}] for {n} atoms; no split")
+            continue
+        out[k] = v
+    return out
+
+
+def fragments_from_splits(offsets, splits) -> np.ndarray:
+    """int32 fragment label per atom for ``Engine.electrostatics``: 0 before the split of its system, 1 from it on; every
+    atom of a system whose split is -1 gets 0 (no pair of that system then counts: its fragment energy is 0)."""
+    offsets = np.asarray(offsets, np.int64)
+    splits = np.asarray(splits, np.int64)
+    sys_of = np.repeat(np.arange(len(splits)), np.diff(offsets))
+    local = np.arange(int(offsets[-1])) - offsets[:-1][sys_of]
+    return ((splits[sys_of] >= 0) & (local >= splits[sys_of])).astype(np.int32)
+
+
 # ------------------------------------------------------------------------------------------------ native ingest
 def _collect(lib, handle):
     import ctypes as C

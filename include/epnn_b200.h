@@ -147,6 +147,44 @@ int epnn_infer_batch_dev(epnn_ctx* ctx, int64_t n_sys, const int32_t* atom_offse
                          const float* xyz_dev, const int32_t* species_dev, const float* Q_dev,
                          const int32_t* npad_host, float* q_out_dev, double* q_out_f64_dev, epnn_stats* stats);
 
+/* Electrostatics of a packed batch of point charges, typically the charges epnn_infer_batch predicted.
+ * (No counterpart in the reference, which stops at the charges; it loads the SSI dimer split <stem>splits.npy,
+ *  charge_gn.py:305-308, but never uses it.)
+ *
+ * Let s be a system, atoms i, j in s, and r_ij = |x_i - x_j|.  Units are e and Angstrom; the C-ABI does no unit
+ * conversion.  The optional `fragment` argument gives an int32 label per atom.  Only equality of labels within one
+ * system matters.
+ * A pair (i, j) is included when all three hold:
+ *   - i != j;
+ *   - r_ij > 0 (coincident atoms are skipped; they contribute nothing);
+ *   - `fragment` is NULL, or fragment_i != fragment_j.
+ * The outputs:
+ *   - phi_i = sum_{j included} q_j / r_ij, the potential at atom i, in e/A.
+ *   - E_s = 1/2 sum_{i in s} q_i phi_i = sum_{i<j included} q_i q_j / r_ij, in e^2/A.  With NULL fragments this is the
+ *     Coulomb energy of the whole system.  With a dimer split it is the inter-monomer energy.
+ *   - mu_s = sum_{i in s} q_i (x_i - c_s), where c_s is the unweighted centroid of the atoms of s, in e*A.  Fragments do
+ *     not change mu.
+ * Everything after loading the float32 coordinates is computed in FP64.  The float32 -> double conversion is exact.
+ *
+ *   atom_offsets   int32[n_sys+1] as in epnn_infer_batch (validated the same way)
+ *   xyz            float32[3*n_atoms]
+ *   q              double[n_atoms], the layout of q_out_f64 of epnn_infer_batch
+ *   fragment       int32[n_atoms] or NULL
+ *   energy_out     double[n_sys] or NULL;  dipole_out double[3*n_sys] (x, y, z per system) or NULL;
+ *   phi_out        double[n_atoms] or NULL.  At least one output must be given.
+ * Every sum has a fixed order and no result is accumulated with atomics: the outputs are bitwise repeatable, and a
+ * system's outputs do not depend on which other systems share the call.  Runs on the ctx's GPU (a sharded ctx too). */
+int epnn_electrostatics(epnn_ctx* ctx, int64_t n_sys, const int32_t* atom_offsets, const float* xyz,
+                        const double* q, const int32_t* fragment, double* energy_out, double* dipole_out,
+                        double* phi_out);
+
+/* Same with DEVICE pointers: atom_offsets stays a HOST array as in epnn_infer_batch_dev, every other pointer is a DEVICE
+ * pointer, so epnn_infer_batch_dev -> epnn_electrostatics_dev chains on the ctx stream with no host copy.  Work is
+ * enqueued on the ctx stream; the call returns after the stream has been synchronised. */
+int epnn_electrostatics_dev(epnn_ctx* ctx, int64_t n_sys, const int32_t* atom_offsets_host, const float* xyz_dev,
+                            const double* q_dev, const int32_t* fragment_dev, double* energy_out_dev,
+                            double* dipole_out_dev, double* phi_out_dev);
+
 /* Neighbour list only (for the bit-exactness check against the reference's is_near mask).
  * Replaces: get_init_edges + the is_near predicate (charge_gn.py:122-163, 90-94).
  *   which = 0: is_near set;  which = 1: the e != 0 set (i != j, D < 3.0).

@@ -142,6 +142,7 @@ inline double __dsub_rn(double a, double b) { return a - b; }
 inline double __dmul_rn(double a, double b) { return a * b; }
 inline double __ddiv_rn(double a, double b) { return a / b; }
 inline double __dsqrt_rn(double a) { return std::sqrt(a); }
+inline double rsqrt(double a) { return 1.0 / std::sqrt(a); }     // the device's FP64 rsqrt is within 1 ulp of this
 inline float __fdiv_rn(float a, float b) { return a / b; }
 inline float __double2float_rn(double a) { return (float)a; }
 
