@@ -49,6 +49,10 @@ SIGNATURES = {
                                       C.c_void_p, C.c_void_p]),
     "epnn_electrostatics_dev": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                           C.c_void_p, C.c_void_p, C.c_void_p]),
+    "epnn_potential_points": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                        C.c_void_p, C.c_void_p]),
+    "epnn_potential_points_dev": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                            C.c_void_p, C.c_void_p, C.c_void_p]),
     "epnn_neighbors": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
                                  C.c_int64, C.POINTER(C.c_int64)]),
     "epnn_init_edges": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]),

@@ -158,6 +158,10 @@ class Model:
         """Energy, dipole and optionally potential of given charges: :meth:`epnn_b200.engine.Engine.electrostatics`."""
         return self._need().electrostatics(offsets, xyz, q, fragment=fragment, potential=potential)
 
+    def potential_points(self, offsets, xyz, q, point_offsets, points, field: bool = False):
+        """Potential and optionally field of given charges at given points: :meth:`epnn_b200.engine.Engine.potential_points`."""
+        return self._need().potential_points(offsets, xyz, q, point_offsets, points, field=field)
+
     def predict_systems(self, systems: Sequence[xyzio.System], npad=None) -> List[np.ndarray]:
         """Charges of parsed systems through the packed path; ``npad`` = pad size N of the reference's dense model
         (default: the largest system, as ``gen_padded_init_state`` pads, charge_gn.py:340)."""

@@ -113,7 +113,8 @@ enum {
     B_XYZ, B_SPECIES, B_OFF, B_Q, B_NPAD, B_ATOMSYS, B_DEG, B_DEGU, B_ROWPTR, B_USTART, B_COL, B_PID, B_PI, B_PJ, B_PD,
     B_E, B_NEAR, B_BUNDLE, B_RGL, B_FARCNT, B_FAROFF, B_FARLIST, B_FAR0CNT, B_FAR0OFF, B_FAR0LIST, B_FAR0W, B_REP, B_ATOMB0, B_BNAT, B_PERM, B_LARGESYS, B_GRID, B_CELLCNT, B_CELLSTART, B_CELLATOMS, B_DTMP, B_H, B_L2, B_S, B_U, B_V, B_DELTA, B_QD, B_SCANTMP, B_CNTL, B_RGLOFF,
     B_OUT32, B_OUT64, B_MISC, B_OFFIN, B_SPTAB, B_SPSTAMP, B_ROWBLK, B_ROWL, B_ARGS, B_DEGALL, B_ACTIVE, B_XYZ_1, B_SPECIES_1, B_Q_1, B_OUT32_1, B_OUT64_1, B_OFFIN_1, B_BPMASK, B_BPTOT, B_BPOFF,
-    B_EL_OFF, B_EL_XYZ, B_EL_Q, B_EL_FRAG, B_EL_E, B_EL_MU, B_EL_PHI, B_EL_PLAN, B_EL_PART, B_COUNT
+    B_EL_OFF, B_EL_XYZ, B_EL_Q, B_EL_FRAG, B_EL_E, B_EL_MU, B_EL_PHI, B_EL_PLAN, B_EL_PART,
+    B_PT_XYZ, B_PT_Q, B_PT_PTS, B_PT_PHI, B_PT_FIELD, B_PT_PLAN, B_PT_PART, B_COUNT
 };
 
 static int fail(epnn_ctx* c, int code, const char* fmt, ...) {
@@ -1065,6 +1066,82 @@ extern "C" int epnn_electrostatics_dev(epnn_ctx* c, int64_t n_sys, const int32_t
                                        const double* q_dev, const int32_t* fragment_dev, double* energy_out_dev,
                                        double* dipole_out_dev, double* phi_out_dev) {
     return elst_impl(c, n_sys, off_host, false, xyz_dev, q_dev, fragment_dev, energy_out_dev, dipole_out_dev, phi_out_dev);
+}
+
+// ------------------------------------------------------------------------------------------------
+// Potential and field of given charges at given points (epnn_elst.cu).  Chunks of elst_pt_chunks run one after the other
+// on the ctx stream, which orders the reuse of every workspace, so the call synchronises once, at the end.
+static int points_impl(epnn_ctx* c, int64_t n_sys, const int32_t* off, bool host_io, const float* xyz, const double* q,
+                       const int64_t* poff, const double* pts, double* phi, double* field) {
+    if (!c) return EPNN_E_INVALID;
+    int rc = validate_offsets(c, n_sys, off);
+    if (rc != EPNN_OK) return rc;
+    if (n_sys > 0 && !poff) return fail(c, EPNN_E_INVALID, "point_offsets is NULL");
+    if (n_sys > 0 && poff[0] != 0) return fail(c, EPNN_E_INVALID, "point_offsets[0] must be 0");
+    for (int64_t s = 0; s < n_sys; ++s)
+        if (poff[s + 1] < poff[s]) return fail(c, EPNN_E_INVALID, "point_offsets decrease at system %lld", (long long)s);
+    if (n_sys == 0) return EPNN_OK;
+    if (!xyz || !q) return fail(c, EPNN_E_INVALID, "NULL input pointer (xyz or q)");
+    if (!phi && !field) return fail(c, EPNN_E_INVALID, "every output pointer is NULL (phi_out, field_out)");
+    if (poff[n_sys] > 0 && !pts) return fail(c, EPNN_E_INVALID, "points is NULL");
+    CU(c, cudaSetDevice(c->device));
+    cudaStream_t st = c->stream;
+    std::vector<ElstPtChunk> chunks;
+    elst_pt_chunks(off, poff, n_sys, c->chunk_atoms, ELST_PT_CHUNK, chunks);
+    std::vector<ElstPtItem> items;
+    std::vector<ElstPtRed> red;
+    void* p;
+    for (const ElstPtChunk& ch : chunks) {
+        const int a0 = off[ch.s0], na = off[ch.s1] - off[ch.s0];
+        const int64_t np = ch.p1 - ch.p0;
+        const long long rows = elst_pt_plan(off, poff, ch, items, red);
+        ElstPtArgs a;
+        const size_t items_bytes = sizeof(ElstPtItem) * items.size(), red_bytes = sizeof(ElstPtRed) * red.size();
+        if ((rc = ensure(c, B_PT_PLAN, items_bytes + red_bytes, &p)) != EPNN_OK) return rc;
+        CU(c, cudaMemcpyAsync(p, items.data(), items_bytes, cudaMemcpyHostToDevice, st));
+        if (!red.empty()) CU(c, cudaMemcpyAsync((char*)p + items_bytes, red.data(), red_bytes, cudaMemcpyHostToDevice, st));
+        a.items = (const ElstPtItem*)p; a.red = (const ElstPtRed*)((char*)p + items_bytes);
+        a.partial = nullptr;
+        if (rows > 0) {
+            if ((rc = ensure(c, B_PT_PART, sizeof(double) * (field ? 4 : 1) * (size_t)rows, &p)) != EPNN_OK) return rc;
+            a.partial = (double*)p;
+        }
+        if (host_io) {
+            if ((rc = ensure(c, B_PT_XYZ, sizeof(float) * 3 * (size_t)na, &p)) != EPNN_OK) return rc;
+            a.xyz = (const float*)p;
+            CU(c, cudaMemcpyAsync(p, xyz + 3 * (size_t)a0, sizeof(float) * 3 * (size_t)na, cudaMemcpyHostToDevice, st));
+            if ((rc = ensure(c, B_PT_Q, sizeof(double) * (size_t)na, &p)) != EPNN_OK) return rc;
+            a.q = (const double*)p;
+            CU(c, cudaMemcpyAsync(p, q + a0, sizeof(double) * (size_t)na, cudaMemcpyHostToDevice, st));
+            if ((rc = ensure(c, B_PT_PTS, sizeof(double) * 3 * (size_t)np, &p)) != EPNN_OK) return rc;
+            a.pts = (const double*)p;
+            CU(c, cudaMemcpyAsync(p, pts + 3 * ch.p0, sizeof(double) * 3 * (size_t)np, cudaMemcpyHostToDevice, st));
+            a.phi = a.field = nullptr;
+            if (phi) { if ((rc = ensure(c, B_PT_PHI, sizeof(double) * (size_t)np, &p)) != EPNN_OK) return rc; a.phi = (double*)p; }
+            if (field) { if ((rc = ensure(c, B_PT_FIELD, sizeof(double) * 3 * (size_t)np, &p)) != EPNN_OK) return rc; a.field = (double*)p; }
+        } else {
+            a.xyz = xyz + 3 * (size_t)a0; a.q = q + a0; a.pts = pts + 3 * ch.p0;
+            a.phi = phi ? phi + ch.p0 : nullptr; a.field = field ? field + 3 * ch.p0 : nullptr;
+        }
+        CU(c, launch_elst_points(a, (int)items.size(), (int)red.size(), st));
+        if (host_io) {
+            if (phi) CU(c, cudaMemcpyAsync(phi + ch.p0, a.phi, sizeof(double) * (size_t)np, cudaMemcpyDeviceToHost, st));
+            if (field) CU(c, cudaMemcpyAsync(field + 3 * ch.p0, a.field, sizeof(double) * 3 * (size_t)np, cudaMemcpyDeviceToHost, st));
+        }
+    }
+    CU(c, cudaStreamSynchronize(st));
+    return EPNN_OK;
+}
+
+extern "C" int epnn_potential_points(epnn_ctx* c, int64_t n_sys, const int32_t* off, const float* xyz, const double* q,
+                                     const int64_t* point_offsets, const double* points, double* phi_out, double* field_out) {
+    return points_impl(c, n_sys, off, true, xyz, q, point_offsets, points, phi_out, field_out);
+}
+
+extern "C" int epnn_potential_points_dev(epnn_ctx* c, int64_t n_sys, const int32_t* off_host, const float* xyz_dev,
+                                         const double* q_dev, const int64_t* point_offsets_host, const double* points_dev,
+                                         double* phi_out_dev, double* field_out_dev) {
+    return points_impl(c, n_sys, off_host, false, xyz_dev, q_dev, point_offsets_host, points_dev, phi_out_dev, field_out_dev);
 }
 
 // ------------------------------------------------------------------------------------------------

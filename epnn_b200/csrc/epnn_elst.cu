@@ -144,11 +144,88 @@ __global__ void __launch_bounds__(ELST_RED) elst_reduce_kernel(const ElstArgs a)
     }
 }
 
+// ---- potential (and field) at given points (epnn_potential_points) ---------------------------------------------------
+// A CTA owns up to ELST_PT_TILE points of one system (one per thread) and streams one source part of that system's atoms
+// through shared memory in tiles of ELST_PT_TILE, in index order.  The parts are fixed slices of ELST_PT_PART atoms, so a
+// point's sums depend only on the point, its system's atoms and charges: not on the other points, the chunking or the GPU.
+// FIELD adds E = sum_j q_j (p - x_j) / r^3; phi-only calls do not carry its accumulators.
+template <bool FIELD>
+__global__ void __launch_bounds__(ELST_PT_TILE) elst_point_kernel(const ElstPtArgs a) {
+    __shared__ ElstSrc src[ELST_PT_TILE];
+    const ElstPtItem it = a.items[blockIdx.x];
+    const int t = (int)threadIdx.x;
+    const long long pi = it.p0 + (t < it.np ? t : it.np - 1);    // threads past the end compute a copy and write nothing
+    const double px = a.pts[3 * pi], py = a.pts[3 * pi + 1], pz = a.pts[3 * pi + 2];
+    double phi = 0.0, ex = 0.0, ey = 0.0, ez = 0.0;
+    for (int j0 = it.s0; j0 < it.s1; j0 += ELST_PT_TILE) {
+        const int m = it.s1 - j0 < ELST_PT_TILE ? it.s1 - j0 : ELST_PT_TILE;
+        __syncthreads();                                          // the previous tile has been read by every thread
+        if (t < m) {
+            const int j = it.a0 + j0 + t;
+            src[t] = ElstSrc{(double)a.xyz[3 * j], (double)a.xyz[3 * j + 1], (double)a.xyz[3 * j + 2], a.q[j]};
+        }
+        __syncthreads();
+#pragma unroll 4
+        for (int k = 0; k < m; ++k) {
+            const ElstSrc s = src[k];
+            const double dx = px - s.x, dy = py - s.y, dz = pz - s.z;
+            const double r2 = dx * dx + dy * dy + dz * dz;
+            const bool in = r2 > 0.0;                             // selects instead of a branch, as in elst_sum
+            const double rinv = rsqrt(in ? r2 : 1.0), qr = (in ? s.q : 0.0) * rinv;
+            phi += qr;
+            if (FIELD) {
+                const double w = qr * rinv * rinv;
+                ex += w * dx; ey += w * dy; ez += w * dz;
+            }
+        }
+    }
+    if (t >= it.np) return;
+    const long long i = it.p0 + t;
+    if (it.pw < 0) {
+        if (a.phi) a.phi[i] = phi;
+        if (FIELD) { a.field[3 * i] = ex; a.field[3 * i + 1] = ey; a.field[3 * i + 2] = ez; }
+    } else if (FIELD) {
+        double* w = a.partial + 4 * (it.pw + t);
+        w[0] = phi; w[1] = ex; w[2] = ey; w[3] = ez;
+    } else {
+        a.partial[it.pw + t] = phi;
+    }
+}
+
+// Adds the parts of the points of a split system in part order.
+template <bool FIELD>
+__global__ void __launch_bounds__(ELST_PT_TILE) elst_point_reduce_kernel(const ElstPtArgs a) {
+    const ElstPtRed r = a.red[blockIdx.x];
+    const int t = (int)threadIdx.x;
+    if (t >= r.np) return;
+    constexpr int W = FIELD ? 4 : 1;
+    double v[W];
+    for (int k = 0; k < W; ++k) v[k] = 0.0;
+    for (int p = 0; p < r.parts; ++p) {
+        const double* w = a.partial + W * (r.pw + (long long)p * r.stride + t);
+        for (int k = 0; k < W; ++k) v[k] += w[k];
+    }
+    const long long i = r.p0 + t;
+    if (a.phi) a.phi[i] = v[0];
+    if (FIELD) { a.field[3 * i] = v[1 % W]; a.field[3 * i + 1] = v[2 % W]; a.field[3 * i + 2] = v[3 % W]; }
+}
+
 #ifndef EPNN_CPU_EMU
 cudaError_t launch_elst(const ElstArgs& a, int n_items, int n_large, cudaStream_t st) {
     if (a.n_sys > 0) elst_small_kernel<<<div_up(a.n_sys, ELST_WARPS), ELST_WARPS * 32, 0, st>>>(a);
     if (n_items > 0) elst_pair_kernel<<<n_items, ELST_TILE, 0, st>>>(a);
     if (n_large > 0) elst_reduce_kernel<<<n_large, ELST_RED, 0, st>>>(a);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_elst_points(const ElstPtArgs& a, int n_items, int n_red, cudaStream_t st) {
+    if (a.field) {
+        if (n_items > 0) elst_point_kernel<true><<<n_items, ELST_PT_TILE, 0, st>>>(a);
+        if (n_red > 0) elst_point_reduce_kernel<true><<<n_red, ELST_PT_TILE, 0, st>>>(a);
+    } else {
+        if (n_items > 0) elst_point_kernel<false><<<n_items, ELST_PT_TILE, 0, st>>>(a);
+        if (n_red > 0) elst_point_reduce_kernel<false><<<n_red, ELST_PT_TILE, 0, st>>>(a);
+    }
     return cudaGetLastError();
 }
 #endif   // !EPNN_CPU_EMU

@@ -349,6 +349,8 @@ cudaError_t launch_atom_const(const Workspace& w, int mode, const StepW<float>* 
                               int h_is_zero, float* q_out, double* q_out64, cudaStream_t st, int* n_launch);   // option pair_const
 struct ElstArgs;
 cudaError_t launch_elst(const ElstArgs& a, int n_items, int n_large, cudaStream_t st);   // epnn_elst.cu (plan: epnn_elst.cuh)
+struct ElstPtArgs;
+cudaError_t launch_elst_points(const ElstPtArgs& a, int n_items, int n_red, cudaStream_t st);   // epnn_elst.cu (plan: epnn_elst.cuh)
 
 #endif   // !EPNN_CPU_EMU
 static inline int div_up(int64_t a, int64_t b) { return (int)((a + b - 1) / b); }

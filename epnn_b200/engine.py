@@ -13,6 +13,7 @@ from .checkpoint import Weights
 # Unit conversions of the electrostatics outputs (the C-ABI works in e and Angstrom)
 COULOMB_KCAL = 332.0637133       # e^2/A -> kcal/mol: e^2 / (4 pi eps0 A) in kcal/mol, CODATA 2018
 DEBYE_PER_E_ANGSTROM = 4.80320471   # e*A -> Debye, CODATA 2018
+BOHR_ANGSTROM = 0.529177210903     # Bohr radius in A, CODATA 2018: phi [e/A] * BOHR_ANGSTROM = phi [e/bohr]
 
 
 def _ptr(a: Optional[np.ndarray]):
@@ -182,6 +183,44 @@ class Engine:
                                                      C.c_void_p(q_dev), C.c_void_p(fragment_dev or None),
                                                      C.c_void_p(energy_dev or None), C.c_void_p(dipole_dev or None),
                                                      C.c_void_p(phi_dev or None)))
+
+    def potential_points(self, offsets, xyz, q, point_offsets, points, field: bool = False):
+        """Potential phi(p) = sum_j q_j / r_pj (e/A) and, with ``field``, E(p) = sum_j q_j (p - x_j) / r_pj^3 (e/A^2) of
+        the charges of each system at its own points, in FP64 on the GPU (epnn_potential_points in include/epnn_b200.h).
+        System s owns the points ``points[point_offsets[s]:point_offsets[s + 1]]`` (a system may have none); atoms at
+        r = 0 from a point are skipped.  Returns ``{"phi": (P,) [, "field": (P, 3)]}`` float64 arrays."""
+        offsets = _as(offsets, np.int32)
+        xyz = _as(xyz, np.float32)
+        q = _as(q, np.float64)
+        poff = _as(point_offsets, np.int64)
+        pts = _as(points, np.float64)
+        n_sys = offsets.shape[0] - 1
+        n_atoms = int(offsets[-1]) if n_sys >= 0 and offsets.size else 0
+        if poff.shape[0] != offsets.shape[0]:
+            raise ValueError("point_offsets must have one entry per system plus one, like atom_offsets")
+        n_pts = int(poff[-1]) if poff.size else 0
+        if xyz.size != 3 * n_atoms or q.size != n_atoms or pts.size != 3 * n_pts:
+            raise ValueError("array sizes are inconsistent with atom_offsets / point_offsets")
+        out = {"phi": np.empty(n_pts, np.float64)}
+        if field:
+            out["field"] = np.empty((n_pts, 3), np.float64)
+        self._check(self.lib.epnn_potential_points(self._h, n_sys, _ptr(offsets), _ptr(xyz), _ptr(q), _ptr(poff),
+                                                   _ptr(pts), _ptr(out["phi"]), _ptr(out.get("field"))))
+        return out
+
+    def potential_points_dev(self, offsets_host, xyz_dev: int, q_dev: int, point_offsets_host, points_dev: int,
+                             phi_dev: int = 0, field_dev: int = 0):
+        """Device-pointer variant of :meth:`potential_points`: the ``*_dev`` arguments are raw CUDA device addresses (ints,
+        0 = NULL); both offset arrays stay on the host.  ``q_dev`` holds float64 charges, e.g. the ``q_out64_dev`` of
+        :meth:`infer_batch_dev`."""
+        offsets_host = _as(offsets_host, np.int32)
+        poff = _as(point_offsets_host, np.int64)
+        n_sys = offsets_host.shape[0] - 1
+        if poff.shape[0] != offsets_host.shape[0]:
+            raise ValueError("point_offsets must have one entry per system plus one, like atom_offsets")
+        self._check(self.lib.epnn_potential_points_dev(self._h, n_sys, _ptr(offsets_host), C.c_void_p(xyz_dev),
+                                                       C.c_void_p(q_dev), _ptr(poff), C.c_void_p(points_dev or None),
+                                                       C.c_void_p(phi_dev or None), C.c_void_p(field_dev or None)))
 
     def neighbors(self, offsets, xyz, which: int = 0):
         """(rowptr, col) CSR of the is_near set (which=0) or the e != 0 set (which=1); global atom indices."""

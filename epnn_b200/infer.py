@@ -41,6 +41,17 @@ def save_electrostatics(path, model, base, stems, offsets, xyz, q64):
              dipole_debye=full["dipole"] * DEBYE_PER_E_ANGSTROM)
 
 
+def save_cubes(directory, model, stems, offsets, xyz, species, n_elems, q64, spacing, margin):
+    """``--cube``: one Gaussian cube file of the potential of the FP64 charges per system, ``DIR/<stem>.cube``."""
+    from . import cube, elements
+    os.makedirs(directory, exist_ok=True)
+    Z = elements.z_table(n_elems)[species]
+    for i, stem in enumerate(stems):
+        a0, a1 = int(offsets[i]), int(offsets[i + 1])
+        cube.esp_cube(os.path.join(directory, stem + ".cube"), model, Z[a0:a1], xyz[a0:a1], q64[a0:a1], spacing, margin,
+                      comment=f"{stem}: epnn_b200 electrostatic potential of the predicted charges")
+
+
 def main(argv=None):
     global model
     ap = argparse.ArgumentParser(description=__doc__, formatter_class=argparse.RawDescriptionHelpFormatter)
@@ -59,9 +70,20 @@ def main(argv=None):
                     help="also save the electrostatics of the predicted FP64 charges (packed path only): names, energy_kcal, "
                          "inter_kcal and q_first_fragment of the two monomers of each <stem>splits.npy dimer (NaN without "
                          "one), split, dipole_debye")
+    ap.add_argument("--cube", default=None, metavar="DIR",
+                    help="also write DIR/<stem>.cube, the electrostatic potential of the predicted FP64 charges of every "
+                         "system on a grid (Gaussian cube: bohr, e/bohr; packed path only).  At the defaults a QM9 "
+                         "molecule gives about 8e4 points, about 1.1 MB (0.6 to 1.6 MB)")
+    ap.add_argument("--cube-spacing", type=float, default=0.3, metavar="A", help="grid spacing of --cube in A (default 0.3)")
+    ap.add_argument("--cube-margin", type=float, default=4.0, metavar="A",
+                    help="space between the atoms and the faces of the --cube grid in A (default 4)")
     args = ap.parse_args(argv)
     if args.elst and args.dense:
         ap.error("--elst needs the packed path (drop --dense)")
+    if args.cube and args.dense:
+        ap.error("--cube needs the packed path (drop --dense)")
+    if not args.cube_spacing > 0 or not args.cube_margin >= 0:
+        ap.error("--cube-spacing must be positive and --cube-margin non-negative")
     options = []
     for kv in args.option:
         k, sep, v = kv.partition("=")
@@ -112,7 +134,7 @@ def main(argv=None):
         q64 = None
         for _ in range(args.repeats):
             timeC = time.time()
-            if args.elst:
+            if args.elst or args.cube:
                 q32, q64 = model.predict_packed(offsets, xyz_all, species_all, Q_all, N, want_f64=True)
                 runs.append(q32)
             else:
@@ -134,6 +156,9 @@ def main(argv=None):
                 y[i, :len(yv), 0] = yv
         if args.elst:
             save_electrostatics(args.elst, model, base, stems, offsets, xyz_all, q64)
+        if args.cube:
+            save_cubes(args.cube, model, stems, offsets, xyz_all, species_all, n_elems, q64, args.cube_spacing,
+                       args.cube_margin)
 
     print(f"avg inference time: {(timeD - timeC) / max(1, args.repeats)}")
     print(f"avg feature time:{(timeB - timeA)}")

@@ -185,6 +185,38 @@ int epnn_electrostatics_dev(epnn_ctx* ctx, int64_t n_sys, const int32_t* atom_of
                             const double* q_dev, const int32_t* fragment_dev, double* energy_out_dev,
                             double* dipole_out_dev, double* phi_out_dev);
 
+/* Electrostatic potential and field of a packed batch of point charges at arbitrary points: an ESP map on a grid, the
+ * potential or field at given sites, or the field at the atoms themselves.
+ *
+ * Let s be a system with atoms j at positions x_j (float32, widened exactly to FP64) and charges q_j (FP64).  Let p be a
+ * point of s (FP64, Angstrom) and r_pj = |p - x_j|.  Atoms with r_pj = 0 are skipped, as coincident atoms are in
+ * epnn_electrostatics.
+ *   - phi(p) = sum_j q_j / r_pj, in e/A.
+ *   - E(p) = -grad phi(p) = sum_j q_j (p - x_j) / r_pj^3, in e/A^2.
+ * Everything after the loads is FP64.  If the points of a system are its own atom coordinates, phi equals the phi_out of
+ * epnn_electrostatics with NULL fragments (to rounding), and q_i E(x_i) is the Coulomb force on atom i at fixed charges.
+ *
+ *   atom_offsets   int32[n_sys+1] as in epnn_infer_batch (validated the same way)
+ *   xyz            float32[3*n_atoms]
+ *   q              double[n_atoms], the layout of q_out_f64 of epnn_infer_batch
+ *   point_offsets  int64[n_sys+1]: system s owns the points [point_offsets[s], point_offsets[s+1]); point_offsets[0] = 0,
+ *                  the offsets do not decrease (a system may have no points)
+ *   points         double[3*n_points] (x, y, z per point); may be NULL only when there are no points
+ *   phi_out        double[n_points] or NULL;  field_out double[3*n_points] (x, y, z per point) or NULL.
+ *                  At least one output must be given.
+ * No result is accumulated with atomics and every sum has a fixed order: the outputs at a point depend only on that
+ * point, its system's atoms and charges, and the build -- not on the system's other points, the other systems, the
+ * chunking of the call or the GPU's SM count.  Runs on the ctx's GPU (a sharded ctx too). */
+int epnn_potential_points(epnn_ctx* ctx, int64_t n_sys, const int32_t* atom_offsets, const float* xyz, const double* q,
+                          const int64_t* point_offsets, const double* points, double* phi_out, double* field_out);
+
+/* Same with DEVICE pointers: atom_offsets and point_offsets stay HOST arrays, every other pointer is a DEVICE pointer, so
+ * epnn_infer_batch_dev -> epnn_potential_points_dev chains on the ctx stream with no host copy.  Work is enqueued on the
+ * ctx stream; the call returns after the stream has been synchronised. */
+int epnn_potential_points_dev(epnn_ctx* ctx, int64_t n_sys, const int32_t* atom_offsets_host, const float* xyz_dev,
+                              const double* q_dev, const int64_t* point_offsets_host, const double* points_dev,
+                              double* phi_out_dev, double* field_out_dev);
+
 /* Neighbour list only (for the bit-exactness check against the reference's is_near mask).
  * Replaces: get_init_edges + the is_near predicate (charge_gn.py:122-163, 90-94).
  *   which = 0: is_near set;  which = 1: the e != 0 set (i != j, D < 3.0).
