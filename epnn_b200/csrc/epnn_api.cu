@@ -14,6 +14,7 @@
 #include "epnn_elst.cuh"
 #include "epnn_internal.cuh"
 #include "epnn_pack.h"
+#include "epnn_plan.h"
 
 #define EPNN_VERSION_STR "epnn_b200 0.1.0 sm_100a"
 
@@ -56,10 +57,6 @@ static const char* load_nccl() {
     return nullptr;
 }
 
-// Equal slices of the atom index space of a batch: rank r owns rows [r * slice, (r + 1) * slice) clipped to n;
-// slice = ceil(n / world) rounded up to 32 rows (all-gathers need equal counts; 32 = the row block of the far kernels).
-static inline int64_t shard_slice_rows(int64_t n, int world) { const int64_t s = (n + world - 1) / world; return (s + 31) / 32 * 32; }
-
 struct epnn_ctx {
     int device = 0, T = 0, n_x = 0, n_species = 0, sm_count = 0;
     cudaStream_t stream = nullptr;           // the stream every kernel / copy of the ctx is enqueued on (own_stream, or the caller's: epnn_set_stream)
@@ -74,20 +71,14 @@ struct epnn_ctx {
     cudaStream_t h2d_stream = nullptr, d2h_stream = nullptr;
     cudaEvent_t ev_h2d[2] = {nullptr, nullptr}, ev_done[2] = {nullptr, nullptr}, ev_d2h[2] = {nullptr, nullptr};
     int precision = 32, timing = 0, keep_hidden = 0;      // precision: 32, 48 (mixed), 64, 0 (auto: probe on the first call)
-    int eff_precision = 32;      // precision of the call in flight (32 / 48 / 64)
     int auto_choice = 0;         // precision chosen by the probe (0 = not probed yet)
     double auto_tol = 2.5e-6;    // a cheaper precision is accepted if its probe charges are within this of the FP64 kernels
     double probe_err32 = -1, probe_err48 = -1;
-    int far_tensor = 2;          // option "gnn_far_tensor": 0 off, 1 on, 2 auto (on when a system of the chunk has >= far_tensor_min atoms)
-    int far_tensor_min = 16384;  // option "gnn_far_tensor_min"
-    int far_tc_impl = 1;         // option "gnn_far_tensor_impl": 1 round-1 kernel (epnn_gnn_tc.cu), 2 warp-specialised (epnn_gnn_tc2.cu)
+    KernelOptions kopt;          // options "pair_const", "pair_tensor", "gnn_far_tensor", "gnn_far_tensor_min", "gnn_far_tensor_impl" (resolve_kernels)
     int dedup_far = 1;           // option "dedup_far": collapse species-equivalent far columns (exact)
-    int pair_tensor = 0;         // option "pair_tensor": EPN bundle kernel on mma.sync 3xTF32 (precision 32 only)
     int fused_prep = 1;          // option "fused_prep": chunks of small systems only build their lists with the two bundle kernels of epnn_bundle_prep.cu
     int atom_tensor = 1;         // option "atom_tensor": FP32 per-atom kernel on mma.sync 3xTF32 (epnn_atom_mma.cu); 0 = the FP32 SIMT warp-tile kernel
     int auto_atom_tensor = 1;    // precision 0 (auto): what the probe decided for the FP32 per-atom kernel
-    int eff_atom_tensor = 1;     // per-atom kernel of the call in flight
-    int pair_const = 2;          // option "pair_const": FP32 kernel set (0 warp-tile, 1 pair-per-thread everywhere, 2 default mix; see epnn_internal.cuh)
     std::vector<float> wf_host;  // host mirror of wf (pair_const passes a step's weights as kernel parameters)
     float* w2split = nullptr;    // [T][2][32][32]: hi / lo parts of W2^T of every message MLP (tensor-core far kernel)
     int shard_rank = 0, shard_world = 1;      // large systems of a call are split over shard_world ranks (epnn_shard_init)
@@ -98,8 +89,7 @@ struct epnn_ctx {
     float* wf = nullptr;         // packed weights, float
     double* wd = nullptr;        // packed weights, double
     std::vector<DevBuf> bufs;    // grow-only workspaces, indexed by enum below
-    std::vector<int2> h_bundles; // host staging of the bundle table of the current chunk
-    std::vector<int> h_large;    // host staging: big systems of the chunk + their cell bases
+    ChunkPlan plan;              // plan of the current chunk (host staging of its bundle, cell and row-block tables)
     int* d_flags = nullptr;      // [0] error bits, [1..4] totals (nnz, P, n_far, n_rg_large)
     int* h_flags = nullptr;      // pinned mirror
     int64_t hidden_atoms = 0;    // atoms covered by the retained hidden state
@@ -288,16 +278,16 @@ extern "C" int epnn_set_option(epnn_ctx* c, const char* key, double value) {
     else if (k == "keep_hidden") c->keep_hidden = value != 0;
     else if (k == "gnn_far_tensor") {
         if (value != 0 && value != 1 && value != 2) return fail(c, EPNN_E_INVALID, "gnn_far_tensor must be 0 (off), 1 (on) or 2 (auto)");
-        c->far_tensor = (int)value;
+        c->kopt.far_tensor = (int)value;
     } else if (k == "gnn_far_tensor_impl") {
         if (value != 1 && value != 2) return fail(c, EPNN_E_INVALID, "gnn_far_tensor_impl must be 1 or 2");
-        c->far_tc_impl = (int)value;
+        c->kopt.far_tensor_impl = (int)value;
     } else if (k == "gnn_far_tensor_min") {
         if (value < SMALL_MAX + 1) return fail(c, EPNN_E_INVALID, "gnn_far_tensor_min must exceed %d", SMALL_MAX);
-        c->far_tensor_min = (int)value;
+        c->kopt.far_tensor_min = (int)value;
     }
     else if (k == "dedup_far") c->dedup_far = value != 0;
-    else if (k == "pair_tensor") c->pair_tensor = value != 0;
+    else if (k == "pair_tensor") c->kopt.pair_tensor = value != 0;
     else if (k == "atom_tensor") c->atom_tensor = value != 0;
     else if (k == "fused_prep") c->fused_prep = value != 0;
     else if (k == "chunk_streams") {
@@ -306,7 +296,7 @@ extern "C" int epnn_set_option(epnn_ctx* c, const char* key, double value) {
     }
     else if (k == "pair_const") {
         if (value != 0 && value != 1 && value != 2) return fail(c, EPNN_E_INVALID, "pair_const must be 0, 1 or 2");
-        c->pair_const = (int)value;
+        c->kopt.pair_const = (int)value;
     }
     else if (k == "chunk_atoms") {
         if (value < 64) return fail(c, EPNN_E_INVALID, "chunk_atoms must be >= 64");
@@ -392,45 +382,36 @@ struct Timer {
     }
 };
 
-// One chunk, device-resident inputs: d_off_in = slice of the caller's GLOBAL offsets (n_sys+1), base = its first value.
-template <typename R>
-static int run_chunk(epnn_ctx* c, int n_sys, int n_atoms, const int32_t* h_off, const int* d_off_in, int base, const float* d_xyz,
-                     const int* d_species, const float* d_Q, const int* d_npad_in, float* d_out32, double* d_out64,
-                     epnn_stats* stats, Timer& tm, int* n_launch, bool neighbors_only, Workspace* ws_out, int slot = 0) {
+// In-place all-gather of an array of pl.rows_pad rows of a sharded chunk: every rank contributes its slice (NCCL on `st`).
+static int gather_rows(epnn_ctx* c, const ChunkPlan& pl, void* buf, size_t row_bytes, cudaStream_t st) {
+    const int rcn = g_nccl.AllGather((char*)buf + (size_t)pl.slice * c->shard_rank * row_bytes, buf, (size_t)pl.slice * row_bytes, /* ncclInt8 */ 0, c->comm, st);
+    if (rcn != 0) return fail(c, EPNN_E_CUDA, "ncclAllGather failed: %s", g_nccl.GetErrorString ? g_nccl.GetErrorString(rcn) : "?");
+    ++c->xchg_calls; c->xchg_bytes += (int64_t)pl.slice * (c->shard_world - 1) * (int64_t)row_bytes;
+    return EPNN_OK;
+}
+
+// Lists of one chunk (plan pl), device-resident inputs: d_off_in = slice of the caller's GLOBAL offsets (n_sys+1), h_off = the
+// same offsets on the host.  Allocates the chunk's list workspaces, launches the list building, synchronises the stream once
+// (totals and error flags) and fills w.  dedup: also build the species tables of the far-column de-duplication.
+static int build_lists(epnn_ctx* c, const KernelChoice& kc, const ChunkPlan& pl, int n_sys, const int32_t* h_off, const int* d_off_in,
+                       const float* d_xyz, const int* d_species, const float* d_Q, const int* d_npad_in, bool dedup,
+                       epnn_stats* stats, Timer& tm, int* n_launch, int slot, Workspace& w) {
     cudaStream_t st = slot ? c->stream2 : c->stream;      // workspace slot 1 belongs to the second chunk stream
     const int sb = slot * B_COUNT;
     int* d_flags = c->d_flags + 8 * slot;
     int* h_flags = c->h_flags + 8 * slot;
-    // mixed precision (48): FP32 pair kernels around an FP64 per-atom kernel (state l2 / h in FP64, S / u / v / delta in FP32)
-    const bool mixed = sizeof(R) == 4 && c->eff_precision == 48;
-    Workspace w;
+    const int base = h_off[0], n_atoms = h_off[n_sys] - h_off[0];
     memset(&w, 0, sizeof(w));
     w.n_atoms = n_atoms; w.n_sys = n_sys; w.sm_count = c->sm_count;
-    // ---- sharded call (epnn_shard_init, world > 1): the rows of the chunk's LARGE systems are split into equal slices of the
-    // atom index space, one per rank; small systems are replicated.  Decided on the host: the offsets are host data.
-    bool has_large = false;
-    for (int s = 0; s < n_sys && !has_large; ++s) has_large = h_off[s + 1] - h_off[s] > SMALL_MAX;
-    const bool sharded = c->shard_world > 1 && c->comm && has_large && !neighbors_only;
-    const int64_t slice = sharded ? shard_slice_rows(n_atoms, c->shard_world) : n_atoms;
-    const int64_t rows_pad = sharded ? slice * c->shard_world : n_atoms;       // exchanged arrays hold world equal slices
-    w.shard_rank = sharded ? c->shard_rank : 0; w.shard_world = sharded ? c->shard_world : 1;
-    w.row_lo = (int)(slice * w.shard_rank < n_atoms ? slice * w.shard_rank : n_atoms);
-    w.row_hi = (int)(slice * (w.shard_rank + 1) < n_atoms ? slice * (w.shard_rank + 1) : n_atoms);
-    // in-place all-gather of an array of rows_pad rows: every rank contributes its slice (NCCL on the ctx stream)
-    auto gather_rows = [&](void* buf, size_t row_bytes) -> int {
-        const int rcn = g_nccl.AllGather((char*)buf + (size_t)slice * w.shard_rank * row_bytes, buf, (size_t)slice * row_bytes, /* ncclInt8 */ 0, c->comm, st);
-        if (rcn != 0) return fail(c, EPNN_E_CUDA, "ncclAllGather failed: %s", g_nccl.GetErrorString ? g_nccl.GetErrorString(rcn) : "?");
-        ++c->xchg_calls; c->xchg_bytes += (int64_t)slice * (w.shard_world - 1) * (int64_t)row_bytes;
-        return EPNN_OK;
-    };
-    w.ek = EKof<R>::v;
+    // sharded call (epnn_shard_init, world > 1): the rows of the chunk's LARGE systems are split into equal slices of the
+    // atom index space, one per rank (pl.row_lo, pl.row_hi); small systems are replicated
+    w.row_lo = pl.row_lo; w.row_hi = pl.row_hi;
+    w.ek = kc.precision == 64 ? ED : EDR;
     w.n_species = c->n_species;
-    w.pair_tensor = c->pair_tensor && sizeof(R) == 4;
-    w.pair_const = sizeof(R) == 4 ? c->pair_const : 0;
-    w.atom_tensor = c->eff_atom_tensor;
+    w.kc = kc;
     w.wf_host = c->wf_host.data(); w.wf_dev = c->wf;
     w.work_counter = d_flags + 7;
-    w.near_counter = stats && !neighbors_only && c->bufs[B_MISC].p ? (unsigned long long*)c->bufs[B_MISC].p : nullptr;
+    w.near_counter = stats && c->bufs[B_MISC].p ? (unsigned long long*)c->bufs[B_MISC].p : nullptr;
     w.slot_counter = stats && c->bufs[B_MISC].p ? (unsigned long long*)c->bufs[B_MISC].p + 2 : nullptr;
     { void* pa; int rca = ensure(c, sb + B_ARGS, 1024, &pa); if (rca != EPNN_OK) return rca; w.args_dev = pa; }
     w.xyz = d_xyz; w.species = d_species; w.Qsys = d_Q;
@@ -455,61 +436,32 @@ static int run_chunk(epnn_ctx* c, int n_sys, int n_atoms, const int32_t* h_off, 
     ENS(B_FAR0CNT, sizeof(int) * ((size_t)n_atoms + 1), far0_cnt, int*);
     ENS(B_FAR0OFF, sizeof(int) * ((size_t)n_atoms + 1), w.far0_off, int*);
     ENS(B_REP, sizeof(int) * ((size_t)n_atoms + 1), w.rep, int*);
-    w.dedup_far = c->dedup_far;
+    w.dedup_far = dedup;
     ENS(B_ATOMB0, sizeof(int) * ((size_t)n_atoms + 1), atom_b0, int*);
     ENS(B_BNAT, sizeof(int) * ((size_t)n_atoms + 1), w.bundle_nat, int*);
-    ENS(B_QD, sizeof(double) * (size_t)rows_pad, w.q, double*);
+    ENS(B_QD, sizeof(double) * (size_t)pl.rows_pad, w.q, double*);
     w.sys_off = off_local; w.npad = npad_local;
 
-    // ---- bundles: greedy runs of consecutive small systems with <= BUNDLE_ATOMS atoms (host: the offsets are host data)
-    {
-        std::vector<int2>& hb = c->h_bundles;
-        hb.clear();
-        int cur0 = -1, cur_n = 0;
-        for (int s = 0; s < n_sys; ++s) {
-            const int a0 = h_off[s] - base, n = h_off[s + 1] - h_off[s];
-            if (n > SMALL_MAX) {
-                if (cur_n) { hb.push_back(make_int2(cur0, cur_n)); cur_n = 0; }
-                continue;
-            }
-            if (cur_n && cur_n + n > BUNDLE_ATOMS) { hb.push_back(make_int2(cur0, cur_n)); cur_n = 0; }
-            if (!cur_n) cur0 = a0;
-            cur_n += n;
-        }
-        if (cur_n) hb.push_back(make_int2(cur0, cur_n));
-        w.n_bundles = (int)hb.size();
-        ENS(B_BUNDLE, sizeof(int2) * (hb.size() + 1), w.bundle, int2*);
-        if (!hb.empty()) CU(c, cudaMemcpyAsync(w.bundle, hb.data(), sizeof(int2) * hb.size(), cudaMemcpyHostToDevice, st));
-    }
+    w.n_bundles = (int)pl.bundles.size();
+    ENS(B_BUNDLE, sizeof(int2) * (pl.bundles.size() + 1), w.bundle, int2*);
+    if (!pl.bundles.empty()) CU(c, cudaMemcpyAsync(w.bundle, pl.bundles.data(), sizeof(int2) * pl.bundles.size(), cudaMemcpyHostToDevice, st));
 
-    // ---- cell lists for the big systems of the chunk (host knows the sizes; budgets give the cell bases without a sync)
+    // ---- cell lists for the big systems of the chunk (the plan's budgets give the cell bases without a sync)
     CellWork cw;
     memset(&cw, 0, sizeof(cw));
-    {
-        std::vector<int>& hl = c->h_large;
-        hl.clear();
-        std::vector<int> base;
-        long long cells = 0, big_atoms = 0;
-        for (int s = 0; s < n_sys; ++s) {
-            const int n = h_off[s + 1] - h_off[s];
-            if (n > CELL_MIN) { hl.push_back(s); base.push_back((int)cells); cells += 4ll * n + 64; big_atoms += n; }
-        }
-        if (cells + 1 >= (1ll << 31)) return fail(c, EPNN_E_UNSUPPORTED, "cell grid exceeds 2^31 cells; lower chunk_atoms");
-        cw.n_large = (int)hl.size(); cw.n_cells = (int)cells;
-        if (cw.n_large) {
-            hl.insert(hl.end(), base.begin(), base.end());
-            int* dl;
-            ENS(B_LARGESYS, sizeof(int) * hl.size(), dl, int*);
-            CU(c, cudaMemcpyAsync(dl, hl.data(), sizeof(int) * hl.size(), cudaMemcpyHostToDevice, st));
-            cw.large_sys = dl; cw.large_base = dl + cw.n_large;
-            ENS(B_GRID, sizeof(CellGrid) * ((size_t)n_sys + 1), cw.grid, CellGrid*);
-            ENS(B_CELLCNT, sizeof(int) * ((size_t)cells + 2), cw.cell_cnt, int*);
-            ENS(B_CELLSTART, sizeof(int) * ((size_t)cells + 2), cw.cell_start, int*);
-            ENS(B_CELLATOMS, sizeof(int) * ((size_t)big_atoms + 1), cw.cell_atoms, int*);
-            int* st2;
-            ENS(B_SCANTMP, sizeof(int) * (((size_t)cells > nmax ? (size_t)cells : nmax) / 1024 + 2), st2, int*);
-            scantmp = st2;
-        }
+    cw.n_large = pl.n_large; cw.n_cells = (int)pl.n_cells;
+    if (cw.n_large) {
+        int* dl;
+        ENS(B_LARGESYS, sizeof(int) * pl.cell_tab.size(), dl, int*);
+        CU(c, cudaMemcpyAsync(dl, pl.cell_tab.data(), sizeof(int) * pl.cell_tab.size(), cudaMemcpyHostToDevice, st));
+        cw.large_sys = dl; cw.large_base = dl + cw.n_large;
+        ENS(B_GRID, sizeof(CellGrid) * ((size_t)n_sys + 1), cw.grid, CellGrid*);
+        ENS(B_CELLCNT, sizeof(int) * ((size_t)pl.n_cells + 2), cw.cell_cnt, int*);
+        ENS(B_CELLSTART, sizeof(int) * ((size_t)pl.n_cells + 2), cw.cell_start, int*);
+        ENS(B_CELLATOMS, sizeof(int) * ((size_t)pl.big_atoms + 1), cw.cell_atoms, int*);
+        int* st2;
+        ENS(B_SCANTMP, sizeof(int) * (((size_t)pl.n_cells > nmax ? (size_t)pl.n_cells : nmax) / 1024 + 2), st2, int*);
+        scantmp = st2;
     }
 
     CU(c, cudaMemsetAsync(d_flags, 0, 8 * sizeof(int), st));
@@ -521,7 +473,7 @@ static int run_chunk(epnn_ctx* c, int n_sys, int n_atoms, const int32_t* h_off, 
     CU(c, launch_prep(w, st, n_launch));
     // Chunks of small systems only (the batched-molecule path): one warp per bundle builds every list from a 48-bit neighbour
     // mask per row (epnn_bundle_prep.cu); chunks with a larger system take the general thread-per-atom kernels.
-    const bool fused = c->fused_prep && !has_large && w.n_bundles > 0;
+    const bool fused = c->fused_prep && !pl.has_large && w.n_bundles > 0;
     BundlePrepWork bw;
     memset(&bw, 0, sizeof(bw));
     if (fused) {
@@ -545,58 +497,19 @@ static int run_chunk(epnn_ctx* c, int n_sys, int n_atoms, const int32_t* h_off, 
     if (h_flags[0] & 1) return fail(c, EPNN_E_INVALID, "npad smaller than the number of atoms for at least one system");
     if (h_flags[0] & 2) return fail(c, EPNN_E_INVALID, "a system with zero (or negative) atoms was passed");
     if (h_flags[0] & 4) return fail(c, EPNN_E_INVALID, "species index outside the element table (n_x=%d has %d species)", c->n_x, c->n_species);
-    w.nnz = h_flags[1]; w.P = h_flags[2]; w.n_far = h_flags[3]; w.n_rg_large = h_flags[4];
+    w.nnz = h_flags[1]; w.P = h_flags[2]; w.n_far = h_flags[3];
     w.n_far0 = (int64_t)(MAX_SPECIES + 1) * n_atoms;      // capacity: at most one slot per species + the pad slot per row
     if (w.nnz < 0 || w.P < 0 || w.n_far < 0) return fail(c, EPNN_E_UNSUPPORTED, "pair lists of one chunk exceed 2^31 entries; lower chunk_atoms");
-    w.nsplit = 1;
-    w.far_tc = 0;
-    w.rg_begin = 0; w.rg_end = w.n_rg_large;
-    if (sharded) {                                   // 4-row groups (numbered over the large systems in order) that overlap [row_lo, row_hi)
-        int g = 0, gb = -1, ge = 0;
-        for (int s = 0; s < n_sys; ++s) {
-            const int a0 = h_off[s] - base, ns_ = h_off[s + 1] - h_off[s];
-            if (ns_ <= SMALL_MAX) continue;
-            for (int i = 0; i < ns_; i += 4, ++g)
-                if (a0 + i + 3 >= w.row_lo && a0 + i < w.row_hi) { if (gb < 0) gb = g; ge = g + 1; }
-        }
-        w.rg_begin = gb < 0 ? 0 : gb; w.rg_end = gb < 0 ? 0 : ge;
-    }
-    if (w.n_rg_large > 0) {
-        int max_n = 0;
-        for (int s = 0; s < n_sys; ++s) max_n = std::max(max_n, h_off[s + 1] - h_off[s]);
-        const bool use_tc = c->far_tensor == 1 || (c->far_tensor == 2 && max_n >= c->far_tensor_min);
-        if (use_tc && sizeof(R) == 4) {              // tensor-core far kernel: CTA units = row group x column range
-            int ns = div_up((int64_t)c->sm_count * 8, w.n_rg_large);
-            ns = ns < 1 ? 1 : (ns > 15 ? 15 : ns);
-            w.far_tc = 1;
-            w.nsplit = ns + 1;                       // + the SIMT kernel's plane (near pairs, pad pair)
-        } else if (c->pair_const && sizeof(R) == 4) {   // experimental row-per-thread far kernel: warp units = 32-row block x column range
-            std::vector<int2> hb;
-            for (int s = 0; s < n_sys; ++s) {
-                const int a0 = h_off[s] - base, ns_ = h_off[s + 1] - h_off[s];
-                if (ns_ > SMALL_MAX) for (int i = 0; i < ns_; i += 32) hb.push_back(make_int2(a0 + i, s));
-            }
-            w.n_rowblk = (int)hb.size();
-            w.blk_begin = 0; w.blk_end = w.n_rowblk;
-            if (sharded) {
-                int bb = -1, be = 0;
-                for (int k = 0; k < w.n_rowblk; ++k)
-                    if (hb[k].x + 31 >= w.row_lo && hb[k].x < w.row_hi) { if (bb < 0) bb = k; be = k + 1; }
-                w.blk_begin = bb < 0 ? 0 : bb; w.blk_end = bb < 0 ? 0 : be;
-            }
-            int2* d_blk;
-            ENS(B_ROWBLK, sizeof(int2) * (hb.size() + 1), d_blk, int2*);
-            CU(c, cudaMemcpyAsync(d_blk, hb.data(), sizeof(int2) * hb.size(), cudaMemcpyHostToDevice, st));
-            CU(c, cudaStreamSynchronize(st));      // hb is a local
-            w.rowblk = d_blk;
-            int ns = div_up((int64_t)c->sm_count * 32, w.n_rowblk);
-            ns = ns < 1 ? 1 : (ns > 15 ? 15 : ns);
-            w.far_tc = 2;
-            w.nsplit = ns + 1;                       // + gnn_pair_kernel's plane (near pairs, pad pair, species slots)
-        } else {
-            int ns = div_up((int64_t)c->sm_count * 64, w.n_rg_large);
-            w.nsplit = ns < 1 ? 1 : (ns > 32 ? 32 : ns);
-        }
+    w.n_rg_large = pl.n_rg_large; w.rg_begin = pl.rg_begin; w.rg_end = pl.rg_end;
+    w.far_kernel = pl.far; w.nsplit = pl.nsplit;
+    if (pl.far == FAR_CONST) {      // row-per-thread far kernel: warp units = 32-row block x column range
+        w.n_rowblk = (int)pl.rowblk.size();
+        w.blk_begin = pl.blk_begin; w.blk_end = pl.blk_end;
+        int2* d_blk;
+        ENS(B_ROWBLK, sizeof(int2) * (pl.rowblk.size() + 1), d_blk, int2*);
+        CU(c, cudaMemcpyAsync(d_blk, pl.rowblk.data(), sizeof(int2) * pl.rowblk.size(), cudaMemcpyHostToDevice, st));
+        CU(c, cudaStreamSynchronize(st));
+        w.rowblk = d_blk;
     }
 
     ENS(B_COL, sizeof(int) * (size_t)(w.nnz + 1), w.col, int*);
@@ -616,15 +529,15 @@ static int run_chunk(epnn_ctx* c, int n_sys, int n_atoms, const int32_t* h_off, 
     ++*n_launch;
     CU(c, cudaGetLastError());
     w.rgl_off = rgl_off;
-    if (w.n_rg_large > 0 && c->dedup_far && !neighbors_only) {      // species tables of the large systems (far-column de-duplication)
+    if (w.n_rg_large > 0 && dedup) {      // species tables of the large systems (far-column de-duplication)
         w.n_sp_tab = w.n_rg_large / 8 + 2;
         ENS(B_SPTAB, sizeof(int) * 32 * (size_t)w.n_sp_tab, w.sp_tab, int*);
         ENS(B_SPSTAMP, sizeof(int) * 2 * (size_t)w.n_sp_tab, w.sp_stamp, int*);
-        if (sharded) {      // the tables' "a row has more than 255 neighbours" flag must come out the same on every rank: full degrees
+        if (pl.sharded) {      // the tables' "a row has more than 255 neighbours" flag must come out the same on every rank: full degrees
             int* dall;
-            ENS(B_DEGALL, sizeof(int) * (size_t)rows_pad, dall, int*);
+            ENS(B_DEGALL, sizeof(int) * (size_t)pl.rows_pad, dall, int*);
             CU(c, cudaMemcpyAsync(dall, w.deg, sizeof(int) * (size_t)n_atoms, cudaMemcpyDeviceToDevice, st));
-            if ((rc = gather_rows(dall, sizeof(int))) != EPNN_OK) return rc;
+            if ((rc = gather_rows(c, pl, dall, sizeof(int), st)) != EPNN_OK) return rc;
             w.deg_all = dall;
         }
         CU(c, launch_sp_tab_build(w, st, n_launch));
@@ -638,26 +551,41 @@ static int run_chunk(epnn_ctx* c, int n_sys, int n_atoms, const int32_t* h_off, 
         if (cw.n_large) ENS(B_DTMP, sizeof(double) * (size_t)(w.nnz + 1), cw.Dtmp, double*);
         CU(c, launch_nbr_fill(w, cw, st, n_launch));
         CU(c, launch_far_fill(w, atom_b0, st, n_launch));
-        if (w.pair_const == 2) CU(c, launch_csr_rowl(w, atom_b0, st, n_launch));
+        if (kc.csr_rowl) CU(c, launch_csr_rowl(w, atom_b0, st, n_launch));
         // species-compressed far list (needs the filled CSR): counts -> offsets -> slots; its size is bounded, no host sync
         CU(c, launch_far0_count(w, far0_cnt, st, n_launch));
         CU(c, launch_scan_i32(far0_cnt, w.far0_off, n_atoms, scantmp, st, n_launch));
         CU(c, launch_far0_fill(w, atom_b0, st, n_launch));
     }
+#undef ENS
     tm.mark(2);
     if (stats) {
         stats->n_pairs_e += w.P;
         stats->n_row_groups += w.n_bundles + w.n_rg_large;
     }
-    if (ws_out) *ws_out = w;
-    if (neighbors_only) return EPNN_OK;
+    return EPNN_OK;
+}
 
+// The T message-passing steps and T electron-passing passes of one chunk whose lists build_lists made (R = float: precision
+// 32 and 48, double: 64).  Enqueued without a host sync.
+template <typename R>
+static int run_layers(epnn_ctx* c, const KernelChoice& kc, const ChunkPlan& pl, Workspace& w, float* d_out32, double* d_out64,
+                      Timer& tm, int* n_launch, int slot) {
+    cudaStream_t st = slot ? c->stream2 : c->stream;
+    const int sb = slot * B_COUNT;
+    const int n_atoms = w.n_atoms;
+    // mixed precision (48): FP32 pair kernels around an FP64 per-atom kernel (state l2 / h in FP64, S / u / v / delta in FP32)
+    const bool mixed = kc.precision == 48;
+    const bool sharded = pl.sharded;
+    void* p;
+    int rc;
+#define ENS(which, bytes, field, type) do { if ((rc = ensure(c, sb + (which), (bytes), &p)) != EPNN_OK) return rc; field = (type)p; } while (0)
     const size_t state_sz = mixed ? sizeof(double) : sizeof(R);
-    ENS(B_H, state_sz * HD * (size_t)rows_pad, w.h, void*);
-    ENS(B_L2, state_sz * HID * (size_t)rows_pad, w.l2, void*);
+    ENS(B_H, state_sz * HD * (size_t)pl.rows_pad, w.h, void*);
+    ENS(B_L2, state_sz * HID * (size_t)pl.rows_pad, w.l2, void*);
     ENS(B_S, sizeof(R) * HID * (size_t)n_atoms * w.nsplit, w.S, void*);
     ENS(B_U, sizeof(R) * HID * (size_t)n_atoms, w.u, void*);
-    ENS(B_V, sizeof(R) * HID * (size_t)rows_pad, w.v, void*);
+    ENS(B_V, sizeof(R) * HID * (size_t)pl.rows_pad, w.v, void*);
     ENS(B_DELTA, sizeof(R) * (size_t)(w.P + 1), w.delta, void*);
 #undef ENS
     CU(c, cudaMemsetAsync(w.h, 0, state_sz * HD * (size_t)n_atoms, st));
@@ -702,8 +630,8 @@ static int run_chunk(epnn_ctx* c, int n_sys, int n_atoms, const int32_t* h_off, 
         CU(c, launch_gnn_bundle<R>(w, msg[t], st, n_launch));
         w.stamp = w.sp_tab ? t + 1 : 0;             // large systems: are this step's v rows equal species by species?
         CU(c, launch_sp_check<R>(w, st, n_launch));
-        if (w.far_tc == 1) {
-            if (c->far_tc_impl == 2)
+        if (w.far_kernel == FAR_TC || w.far_kernel == FAR_TC2) {
+            if (w.far_kernel == FAR_TC2)
                 CU(c, launch_gnn_far_tc2(w, c->w2split + (size_t)t * 2048, c->w2split + (size_t)t * 2048 + 1024, (const float*)msg[t].b2,
                                          w.nsplit - 1, st, n_launch));
             else
@@ -711,7 +639,7 @@ static int run_chunk(epnn_ctx* c, int n_sys, int n_atoms, const int32_t* h_off, 
                                         w.nsplit - 1, st, n_launch));
         }
         if constexpr (sizeof(R) == 4) {
-            if (w.far_tc == 2) CU(c, launch_gnn_far_const(w, msg[t], w.nsplit - 1, st, n_launch));
+            if (w.far_kernel == FAR_CONST) CU(c, launch_gnn_far_const(w, msg[t], w.nsplit - 1, st, n_launch));
         }
         CU(c, launch_gnn_pair<R>(w, msg[t], st, n_launch));
         tm.mark(3);
@@ -720,11 +648,11 @@ static int run_chunk(epnn_ctx* c, int n_sys, int n_atoms, const int32_t* h_off, 
             CU(c, atom(ATOM_UPDATE | ATOM_PROJECT | (t == 0 ? ATOM_FIRST : 0) | (last ? ATOM_WRITE_H : 0), t, t + 1, 0, nullptr, nullptr, 0));
         } else if (!last) {
             CU(c, atom(ATOM_UPDATE | ATOM_PROJECT | (t == 0 ? ATOM_FIRST : 0), t, t + 1, 0, nullptr, nullptr, own));
-            if ((rc = gather_rows(w.v, sizeof(R) * HID)) != EPNN_OK) return rc;
+            if ((rc = gather_rows(c, pl, w.v, sizeof(R) * HID, st)) != EPNN_OK) return rc;
         } else {
             CU(c, atom(ATOM_UPDATE | ATOM_WRITE_H | (t == 0 ? ATOM_FIRST : 0), t, -1, 0, nullptr, nullptr, own));
-            if ((rc = gather_rows(w.l2, state_row)) != EPNN_OK) return rc;
-            if (c->keep_hidden && (rc = gather_rows(w.h, state_row / HID * HD)) != EPNN_OK) return rc;
+            if ((rc = gather_rows(c, pl, w.l2, state_row, st)) != EPNN_OK) return rc;
+            if (c->keep_hidden && (rc = gather_rows(c, pl, w.h, state_row / HID * HD, st)) != EPNN_OK) return rc;
             CU(c, atom(ATOM_PROJECT, -1, c->T, 0, nullptr, nullptr, act));
         }
         tm.mark(!last ? 4 : 6);
@@ -740,28 +668,15 @@ static int run_chunk(epnn_ctx* c, int n_sys, int n_atoms, const int32_t* h_off, 
             else CU(c, atom(ATOM_QUPDATE | ATOM_OUTPUT, -1, -1, 0, d_out32, d_out64, 0));
         } else {
             CU(c, atom(ATOM_QUPDATE, -1, -1, 0, nullptr, nullptr, own));
-            if ((rc = gather_rows(w.q, sizeof(double))) != EPNN_OK) return rc;
+            if ((rc = gather_rows(c, pl, w.q, sizeof(double), st)) != EPNN_OK) return rc;
             if (!last) CU(c, atom(ATOM_PROJECT, -1, c->T + t + 1, 0, nullptr, nullptr, act));
             else CU(c, atom(ATOM_OUTPUT, -1, -1, 0, d_out32, d_out64, 0));
         }
         tm.mark(6);
     }
     c->hidden_atoms = n_atoms;
-    c->hidden_precision = (sizeof(R) == 4 && !mixed) ? 32 : 64;
+    c->hidden_precision = kc.precision == 32 ? 32 : 64;
     return EPNN_OK;
-}
-
-// Splits [0, n_sys) into chunks of at most chunk_atoms atoms (a single larger system gets its own chunk).
-static void plan_chunks(const int32_t* off, int64_t n_sys, int64_t chunk_atoms, std::vector<int64_t>& bounds) {
-    bounds.clear();
-    bounds.push_back(0);
-    int64_t s = 0;
-    while (s < n_sys) {
-        int64_t e = s + 1;
-        while (e < n_sys && (int64_t)off[e + 1] - off[s] <= chunk_atoms) ++e;
-        bounds.push_back(e);
-        s = e;
-    }
 }
 
 static int validate_offsets(epnn_ctx* c, int64_t n_sys, const int32_t* off) {
@@ -774,8 +689,8 @@ static int validate_offsets(epnn_ctx* c, int64_t n_sys, const int32_t* off) {
 }
 
 
-static int infer_impl(epnn_ctx* c, int64_t n_sys, const int32_t* off, bool host_io, const float* xyz, const int32_t* species,
-                      const float* Q, const int32_t* npad_host, float* q_out, double* q_out64, epnn_stats* stats);
+static int infer_impl(epnn_ctx* c, int precision, int atom_tensor, int64_t n_sys, const int32_t* off, bool host_io, const float* xyz,
+                      const int32_t* species, const float* Q, const int32_t* npad_host, float* q_out, double* q_out64, epnn_stats* stats);
 
 // "precision" 0 (auto): run a bounded prefix of the first call through the FP32, mixed and FP64 kernels and keep the cheapest
 // precision whose charges stay within auto_tol of the FP64 kernels (which agree with the float64 oracle to 1e-9).  The
@@ -812,8 +727,7 @@ static int probe_precision(epnn_ctx* c, int64_t n_sys, const int32_t* off, bool 
     const int atom_tensor = c->atom_tensor;
     auto run = [&](int prec, int tensor, std::vector<double>& out) {
         out.resize((size_t)na);
-        c->precision = prec; c->atom_tensor = tensor;
-        return infer_impl(c, ns, off, true, px, ps, pq, npad_host, tmp.data(), out.data(), nullptr);
+        return infer_impl(c, prec, tensor, ns, off, true, px, ps, pq, npad_host, tmp.data(), out.data(), nullptr);
     };
     auto dist = [&]() { double e = 0; for (int64_t i = 0; i < na; ++i) e = fmax(e, fabs(q[1][i] - q[0][i])); return e; };
     int rc = run(64, 0, q[0]);
@@ -827,27 +741,26 @@ static int probe_precision(epnn_ctx* c, int64_t n_sys, const int32_t* off, bool 
     if (rc == EPNN_OK && choice == 64) {
         if ((rc = run(48, 0, q[1])) == EPNN_OK) { c->probe_err48 = dist(); if (c->probe_err48 <= c->auto_tol) choice = 48; }
     }
-    c->precision = 0; c->atom_tensor = atom_tensor;
     c->hidden_atoms = hidden_atoms;
     if (rc != EPNN_OK) return rc;
     c->auto_choice = choice; c->auto_atom_tensor = tensor;
     return EPNN_OK;
 }
 
-static int infer_impl(epnn_ctx* c, int64_t n_sys, const int32_t* off, bool host_io, const float* xyz, const int32_t* species,
-                      const float* Q, const int32_t* npad_host, float* q_out, double* q_out64, epnn_stats* stats) {
-    if (!c) return EPNN_E_INVALID;
+// precision 32 / 48 / 64 with the FP32 per-atom kernel on the tensor path or not (atom_tensor), or 0: the ctx's auto choice
+// (probed on first use)
+static int infer_impl(epnn_ctx* c, int precision, int atom_tensor, int64_t n_sys, const int32_t* off, bool host_io, const float* xyz,
+                      const int32_t* species, const float* Q, const int32_t* npad_host, float* q_out, double* q_out64, epnn_stats* stats) {
     int rc = validate_offsets(c, n_sys, off);
     if (rc != EPNN_OK) return rc;
     if (stats) memset(stats, 0, sizeof(*stats));
     if (n_sys == 0) return EPNN_OK;
     if (!xyz || !species || !Q || (!q_out && !q_out64)) return fail(c, EPNN_E_INVALID, "NULL input/output pointer");
-    if (c->precision == 0 && c->auto_choice == 0) {
-        rc = probe_precision(c, n_sys, off, host_io, xyz, species, Q, npad_host);
-        if (rc != EPNN_OK) return rc;
+    if (precision == 0) {
+        if (c->auto_choice == 0 && (rc = probe_precision(c, n_sys, off, host_io, xyz, species, Q, npad_host)) != EPNN_OK) return rc;
+        precision = c->auto_choice; atom_tensor = c->auto_atom_tensor;
     }
-    c->eff_precision = c->precision == 0 ? c->auto_choice : c->precision;
-    c->eff_atom_tensor = c->precision == 0 ? c->auto_atom_tensor : c->atom_tensor;
+    const KernelChoice kc = resolve_kernels(precision, atom_tensor, c->kopt);
     CU(c, cudaSetDevice(c->device));
     cudaStream_t st = c->stream;
     std::vector<int64_t> bounds;
@@ -927,13 +840,17 @@ static int infer_impl(epnn_ctx* c, int64_t n_sys, const int32_t* off, bool host_
         }
         tmc.mark(1);
         Workspace w;
-        if (c->eff_precision == 64)
-            rc = run_chunk<double>(c, ns, na, off + s0, d_off, a0, d_xyz, d_species, d_Q, d_npad_in, d_o32, d_o64, stats, tmc, &n_launch, false, &w, ws);
+        ChunkPlan& pl = c->plan;
+        if (!plan_chunk(off + s0, ns, c->sm_count, c->shard_rank, c->comm ? c->shard_world : 1, kc, pl))
+            rc = fail(c, EPNN_E_UNSUPPORTED, "cell grid exceeds 2^31 cells; lower chunk_atoms");
         else
-            rc = run_chunk<float>(c, ns, na, off + s0, d_off, a0, d_xyz, d_species, d_Q, d_npad_in, d_o32, d_o64, stats, tmc, &n_launch, false, &w, ws);
+            rc = build_lists(c, kc, pl, ns, off + s0, d_off, d_xyz, d_species, d_Q, d_npad_in, c->dedup_far, stats, tmc, &n_launch, ws, w);
+        if (rc == EPNN_OK)
+            rc = kc.precision == 64 ? run_layers<double>(c, kc, pl, w, d_o32, d_o64, tmc, &n_launch, ws)
+                                    : run_layers<float>(c, kc, pl, w, d_o32, d_o64, tmc, &n_launch, ws);
         if (rc != EPNN_OK) { cudaStreamSynchronize(c->h2d_stream); cudaStreamSynchronize(down); cudaStreamSynchronize(c->stream2); cudaStreamSynchronize(st); return rc; }
         if (piped) {
-            // run_chunk returned after its one host sync (neighbour count): chunk ci - 1 is complete, the bulk of chunk ci is
+            // build_lists made the chunk's one host sync (neighbour count): chunk ci - 1 is complete, the bulk of chunk ci is
             // queued.  Its results go down on their own stream; the other slot is free for chunk ci + 1 once ITS download is done.
             CU(c, cudaEventRecord(c->ev_done[k], cs));
             CU(c, cudaStreamWaitEvent(down, c->ev_done[k], 0));
@@ -967,9 +884,9 @@ static int infer_impl(epnn_ctx* c, int64_t n_sys, const int32_t* off, bool host_
         stats->n_gnn_near_slots = (int64_t)nn[2]; stats->n_gnn_far_slots = (int64_t)nn[3];
         stats->n_systems = n_sys; stats->n_atoms = off[n_sys]; stats->n_chunks = (int64_t)bounds.size() - 1;
         stats->n_launches = n_launch;
-        stats->precision_used = c->eff_precision;
+        stats->precision_used = kc.precision;
         stats->probe_err32 = (float)c->probe_err32; stats->probe_err48 = (float)c->probe_err48;
-        stats->atom_tensor_used = c->eff_precision == 32 ? c->eff_atom_tensor : 0;
+        stats->atom_tensor_used = kc.precision == 32 ? atom_tensor : 0;
     }
     tm.finish(stats);
     tm2.finish(stats);          // (two chunk streams: the phase times of both are added up; they overlap in wall-clock time)
@@ -979,13 +896,15 @@ static int infer_impl(epnn_ctx* c, int64_t n_sys, const int32_t* off, bool host_
 
 extern "C" int epnn_infer_batch(epnn_ctx* c, int64_t n_sys, const int32_t* off, const float* xyz, const int32_t* species,
                                 const float* Q, const int32_t* npad, float* q_out, double* q_out64, epnn_stats* stats) {
-    return infer_impl(c, n_sys, off, true, xyz, species, Q, npad, q_out, q_out64, stats);
+    if (!c) return EPNN_E_INVALID;
+    return infer_impl(c, c->precision, c->atom_tensor, n_sys, off, true, xyz, species, Q, npad, q_out, q_out64, stats);
 }
 
 extern "C" int epnn_infer_batch_dev(epnn_ctx* c, int64_t n_sys, const int32_t* off_host, const float* xyz_dev,
                                     const int32_t* species_dev, const float* Q_dev, const int32_t* npad_host,
                                     float* q_out_dev, double* q_out64_dev, epnn_stats* stats) {
-    return infer_impl(c, n_sys, off_host, false, xyz_dev, species_dev, Q_dev, npad_host, q_out_dev, q_out64_dev, stats);
+    if (!c) return EPNN_E_INVALID;
+    return infer_impl(c, c->precision, c->atom_tensor, n_sys, off_host, false, xyz_dev, species_dev, Q_dev, npad_host, q_out_dev, q_out64_dev, stats);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1161,6 +1080,7 @@ extern "C" int epnn_neighbors(epnn_ctx* c, int64_t n_sys, const int32_t* off, co
     plan_chunks(off, n_sys, c->chunk_atoms, bounds);
     Timer tm{false, st, {}, {}};
     int n_launch = 0;
+    const KernelChoice kc = resolve_kernels(32, c->atom_tensor, c->kopt);
     int64_t written = 0;
     bool overflow = false;
     std::vector<int> h_rowptr, h_col, h_pid;
@@ -1180,7 +1100,8 @@ extern "C" int epnn_neighbors(epnn_ctx* c, int64_t n_sys, const int32_t* off, co
         CU(c, cudaMemsetAsync(bs, 0, sizeof(int) * (size_t)na, st));
         CU(c, cudaMemsetAsync(bq, 0, sizeof(float) * (size_t)ns, st));
         Workspace w;
-        rc = run_chunk<float>(c, ns, na, off + s0, d_off, a0, bx, bs, bq, nullptr, nullptr, nullptr, nullptr, tm, &n_launch, true, &w);
+        if (!plan_chunk(off + s0, ns, c->sm_count, 0, 1, kc, c->plan)) return fail(c, EPNN_E_UNSUPPORTED, "cell grid exceeds 2^31 cells; lower chunk_atoms");
+        rc = build_lists(c, kc, c->plan, ns, off + s0, d_off, bx, bs, bq, nullptr, false, nullptr, tm, &n_launch, 0, w);
         if (rc != EPNN_OK) return rc;
         h_rowptr.resize((size_t)na + 1); h_col.resize((size_t)w.nnz + 1); h_pid.resize((size_t)w.nnz + 1); h_near.resize((size_t)w.P + 1);
         CU(c, cudaMemcpyAsync(h_rowptr.data(), w.rowptr, sizeof(int) * ((size_t)na + 1), cudaMemcpyDeviceToHost, st));

@@ -265,8 +265,9 @@ template <typename R, typename IO>
 cudaError_t launch_atom_io(const Workspace& w, int mode, const StepW<R>* prev, const UpdW<R>* upd, const StepW<R>* next,
                            int h_is_zero, float* q_out, double* q_out64, cudaStream_t st, int* nl, int scope) {
     if (w.n_atoms == 0) return cudaSuccess;
+    const AtomKernel k = scope ? w.kc.atom_scoped : w.kc.atom;
     if constexpr (sizeof(R) == 4) {
-        if (w.pair_const == 1 && scope == 0) return launch_atom_const(w, mode, prev, upd, next, h_is_zero, q_out, q_out64, st, nl);   // experimental (epnn_atom_const.cu)
+        if (k == ATOM_K_CONST) return launch_atom_const(w, mode, prev, upd, next, h_is_zero, q_out, q_out64, st, nl);   // experimental (epnn_atom_const.cu)
     }
     constexpr int NW = sizeof(R) == 4 ? ATOM_NW : 4;
     AtomArgs<R, IO> aa;
@@ -280,7 +281,7 @@ cudaError_t launch_atom_io(const Workspace& w, int mode, const StepW<R>* prev, c
     aa.u = (IO*)w.u; aa.v = (IO*)w.v; aa.q_out = q_out; aa.q_out64 = q_out64;
     aa.scope = scope; aa.row_lo = w.row_lo; aa.row_hi = w.row_hi; aa.active = w.active;
     if constexpr (sizeof(R) == 4 && sizeof(IO) == 4) {       // FP32 calls: launches with a dense layer run on the warp-level tensor path
-        if (w.atom_tensor && ((mode & ATOM_UPDATE) || ((mode & ATOM_PROJECT) && !h_is_zero))) return launch_atom_mma(w, aa, st, nl);
+        if (k == ATOM_K_MMA && ((mode & ATOM_UPDATE) || ((mode & ATOM_PROJECT) && !h_is_zero))) return launch_atom_mma(w, aa, st, nl);
     }
     const size_t smem = sizeof(R) * (ATOM_W_UPD + ATOM_W_PROJ + (size_t)NW * ATOM_TILE + NW * 64) + sizeof(int) * NW * 64;
     cudaError_t e = cudaFuncSetAttribute(scope ? atom_kernel<R, NW, IO, true> : atom_kernel<R, NW, IO, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);

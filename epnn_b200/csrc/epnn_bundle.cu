@@ -440,15 +440,15 @@ static cudaError_t launch_bundle(const Workspace& w, const StepW<R>& sw, cudaStr
 #ifndef EPNN_CPU_EMU
 template <typename R> cudaError_t launch_gnn_bundle(const Workspace& w, const StepW<R>& sw, cudaStream_t st, int* nl) {
     if constexpr (sizeof(R) == 4) {
-        if (w.pair_const == 2) return launch_gnn_bundle_run(w, sw, st, nl);    // row-run mapping (epnn_bundle_run.cu): FP32 default
-        if (w.pair_const == 1) return launch_gnn_bundle_const(w, sw, st, nl);  // pair-per-thread variant with transpose (epnn_bundle_const.cu)
+        if (w.kc.gnn == GNN_RUN) return launch_gnn_bundle_run(w, sw, st, nl);      // row-run mapping (epnn_bundle_run.cu): FP32 default
+        if (w.kc.gnn == GNN_CONST) return launch_gnn_bundle_const(w, sw, st, nl);  // pair-per-thread variant with transpose (epnn_bundle_const.cu)
     }
     return launch_bundle<R, false>(w, sw, st, nl);
 }
 template <typename R> cudaError_t launch_epn_bundle(const Workspace& w, const StepW<R>& sw, cudaStream_t st, int* nl) {
     if constexpr (sizeof(R) == 4) {
-        if (w.pair_tensor) return launch_epn_bundle_mma(w, sw, st, nl);      // optional 3xTF32 mma.sync variant (epnn_bundle_mma.cu)
-        if (w.pair_const) return launch_epn_bundle_const(w, sw, st, nl);     // pair-per-thread variant (epnn_bundle_const.cu): FP32 default
+        if (w.kc.epn == EPN_MMA) return launch_epn_bundle_mma(w, sw, st, nl);       // optional 3xTF32 mma.sync variant (epnn_bundle_mma.cu)
+        if (w.kc.epn == EPN_CONST) return launch_epn_bundle_const(w, sw, st, nl);   // pair-per-thread variant (epnn_bundle_const.cu): FP32 default
     }
     return launch_bundle<R, true>(w, sw, st, nl);
 }
@@ -605,7 +605,7 @@ __global__ void tile_perm_kernel(int64_t P, const int* __restrict__ pair_i, cons
 #ifndef EPNN_CPU_EMU
 cudaError_t launch_tile_perm(const Workspace& w, const int* atom_b0, cudaStream_t st, int* nl) {
     if (w.n_atoms == 0 || w.n_bundles == 0) return cudaSuccess;
-    if (w.P > 0 && !(w.pair_const == 2 && w.ek == EDR)) {      // only the round-1 warp-tile GNN kernel reads perm_j
+    if (w.P > 0 && w.kc.tile_perm) {
         tile_perm_kernel<<<div_up(w.P, 256), 256, 0, st>>>(w.P, w.pair_i, w.pair_j, w.atom_sys, w.sys_off, atom_b0,
                                                            w.ustart, w.bundle_nat, w.perm_j);
         ++*nl;

@@ -309,8 +309,9 @@ cudaError_t launch_gnn_pair(const Workspace& w, const StepW<R>& sw, cudaStream_t
     cudaError_t e = cudaSuccess;
     if (w.n_rg_large > 0) {      // small systems (n <= SMALL_MAX) are handled by the bundle kernel (epnn_bundle.cu)
         // tensor-core mode: this kernel does the near pairs + pad pair only (one unit per row group, last plane)
-        const int ns = w.far_tc ? 1 : w.nsplit;
-        ga.skip_far = w.far_tc; ga.plane = w.far_tc ? w.nsplit - 1 : 0;
+        const int skip_far = w.far_kernel != FAR_SIMT;
+        const int ns = skip_far ? 1 : w.nsplit;
+        ga.skip_far = skip_far; ga.plane = skip_far ? w.nsplit - 1 : 0;
         // sharded call: the row groups that overlap this rank's slice (rows of a boundary group that lie outside it are computed
         // from whatever their u row holds and never read: S is only consumed for owned rows)
         ga.rg_atom = w.rg_large; ga.nsplit = ns;

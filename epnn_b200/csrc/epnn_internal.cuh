@@ -13,6 +13,7 @@
 #include "../../include/epnn_b200.h"
 
 #include "epnn_consts.h"
+#include "epnn_plan.h"
 
 // ------------------------------------------------------------------------------------------------
 // Vector of 4 reals: one LDS.128 / LDG.128 for float, two for double.
@@ -238,10 +239,8 @@ struct Workspace {
     int* far0_off; unsigned short* far0_list; unsigned char* far0_w; int* rep; int64_t n_far0; int dedup_far;   // species-compressed far list   // per-bundle list of the GNN's e == 0 ("far") ordered pairs
     int* rg_large; int n_rg_large; int nsplit;    // 4-row groups of the large systems
     const int2* rowblk; int n_rowblk;             // 32-row blocks of the large systems (first atom, system): units of gnn_far_const_kernel
-    int far_tc;                                   // 1: the far part of the big-system message sum runs on the tensor cores (2: on the
-                                                  //    experimental row-per-thread FP32 kernel, epnn_gnn_far_const.cu);
-                                                  //    planes [0, nsplit-1) of S are theirs, the SIMT kernel (near only) owns the last
-    int shard_rank, shard_world;                  // sharded call (epnn_shard_init): large systems are split by rows over the ranks
+    FarKernel far_kernel;                         // far part of the big-system message sum (ChunkPlan::far); unless FAR_SIMT, planes
+                                                  // [0, nsplit-1) of S are the far kernel's, the SIMT kernel (near only) owns the last
     int row_lo, row_hi;                           // rows [row_lo, row_hi) of the chunk belong to this rank (unsharded: [0, n_atoms))
     int rg_begin, rg_end, blk_begin, blk_end;     // 4-row groups / 32-row blocks of the large systems that overlap the slice
     const unsigned char* active;                  // sharded: 1 for owned atoms and their near neighbours (rows whose projections are needed here)
@@ -252,10 +251,7 @@ struct Workspace {
     int* sp_stamp;                                // [n_sp_tab][2]: stamp of the last step whose v rows were NOT species-wise equal | dedup forbidden
     int stamp;                                    // stamp of the current message-passing step (t + 1); 0 = de-duplication off
     int n_species;                                // species of the element table in use (8 or 9)
-    int pair_tensor;                              // 1: electron-passing bundle kernel on the warp-level tensor path (3xTF32, FP32 only)
-    int pair_const;                               // FP32 kernel set: 0 warp-tile kernels (round 1), 1 pair-per-thread kernels everywhere,
-                                                  // 2 (default) row-run GNN bundle kernel + pair-per-thread EPN bundle kernel + row-per-thread far kernel
-    int atom_tensor;                              // 1 (default): FP32 per-atom kernel on the warp-level tensor path (3xTF32, epnn_atom_mma.cu)
+    KernelChoice kc;                              // kernels of the call (resolve_kernels)
     void* args_dev;                               // 1 KB device scratch: argument block of the kernels that take theirs through global memory
     const float* wf_host; const float* wf_dev;    // packed FP32 weights: host mirror and device base (pair_const passes weights as kernel parameters)
     unsigned long long* near_counter;             // device counter (statistics, may be NULL): unordered pairs in the is_near set
@@ -295,7 +291,7 @@ cudaError_t upload_rbf_centers(const double* mu);
 cudaError_t upload_rbf_basis(const double* B);      // [ED][EDR]
 
 cudaError_t launch_edge_desc(const Workspace& w, cudaStream_t st, int* n_launch, bool gather);   // descriptors + near flags of the pair list (gather: D from the coordinates)
-cudaError_t launch_tile_perm(const Workspace& w, const int* atom_b0, cudaStream_t st, int* n_launch);   // only the round-1 GNN bundle kernel needs it
+cudaError_t launch_tile_perm(const Workspace& w, const int* atom_b0, cudaStream_t st, int* n_launch);   // if w.kc.tile_perm
 cudaError_t launch_bundle_prep_count(const Workspace& w, const BundlePrepWork& bw, int* scantmp, int* flags, cudaStream_t st, int* n_launch);
 cudaError_t launch_bundle_prep_fill(const Workspace& w, const BundlePrepWork& bw, cudaStream_t st, int* n_launch);
 cudaError_t launch_far_count(const Workspace& w, int* far_cnt, int* atom_b0, cudaStream_t st, int* n_launch);

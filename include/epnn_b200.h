@@ -105,7 +105,7 @@ const char* epnn_last_error(const epnn_ctx* ctx);
  * tensor kernel is 1.5x the FP32 SIMT one;
  * "pair_tensor" 0 (default) / 1: systems with at most 48 atoms evaluate the electron-passing pair MLP on the warp-level
  * tensor path (mma.sync m16n8k8 TF32 inputs, 3xTF32 split, FP32 accumulation, operands chained through registers)
- * instead of FP32 SIMT (precision 32 only; per-pair transfers differ from the SIMT path by about 1e-6 relative);
+ * instead of FP32 SIMT (FP32 / mixed precision only; per-pair transfers differ from the SIMT path by about 1e-6 relative);
  * "atom_tensor" 1 (default) / 0: FP32 calls run the dense layers of the per-atom kernel (folded update MLP, first-layer
  * projections: GEMMs over all atoms of a chunk) on the warp-level tensor path, 3xTF32 split with FP32 accumulation
  * (epnn_atom_mma.cu), which leaves that kernel bound by its HBM traffic; 0 = the FP32 SIMT warp-tile kernel.  Same

@@ -1,7 +1,7 @@
 """Large-system message kernels against the scalable float64 oracle (oracle/epnn_oracle_sparse.py, torch on the GPU).
 
 Systems above 48 atoms sum the GNN messages over all pairs with one of three kernels, each of which cuts a system's
-columns into ``ns`` ranges (epnn_api.cu, run_chunk):
+columns into ``ns`` ranges (epnn_plan.h, plan_chunk):
 
   * tcgen05 (epnn_gnn_tc.cu / epnn_gnn_tc2.cu, FP32): ns = clamp(ceil(8 SM / n_rg), 1, 15), n_rg = sum ceil(n_s / 4),
     range length rounded up to 128; on by default once a system of the chunk has >= 16 384 atoms ("gnn_far_tensor_min");

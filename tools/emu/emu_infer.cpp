@@ -1,12 +1,12 @@
 // CPU emulation of a WHOLE charge inference through the product's own kernels (test infrastructure; see cuda_emu.h).
 //
-// Weights are packed / folded by the product's own host code (epnn_pack.h, the code epnn_create runs); then the kernels
-// of epnn_neighbor / epnn_bundle / epnn_gnn / epnn_epn / epnn_atom (and, with variant = 1, epnn_bundle_const /
-// epnn_atom_const; with variant = 2, the mma.sync electron-passing kernel epnn_bundle_mma; with variant = 3, the shipped
-// FP32 set of "pair_const" 2: the row-run GNN bundle kernel epnn_bundle_run, the electron-passing kernel of
-// epnn_bundle_const and the far_const kernel for large systems, with the SIMT per-atom kernel) run in the launch order of
-// run_chunk (epnn_api.cu), FP32, one chunk.  The only code that is not the product's is this orchestration (a
-// restatement of run_chunk without streams and workspaces) and two host-side scans.
+// Weights are packed / folded by the product's own host code (epnn_pack.h, the code epnn_create runs); the chunk plan and
+// the kernel choice are the library's (epnn_plan.h: plan_chunk, resolve_kernels for precision 32 with the options of the
+// variant, "atom_tensor" 0 and "gnn_far_tensor" 0); then the kernels of epnn_neighbor / epnn_bundle /
+// epnn_bundle_const / epnn_bundle_run / epnn_bundle_mma / epnn_gnn / epnn_gnn_far_const / epnn_epn / epnn_atom /
+// epnn_atom_const that the choice names run in the launch order of build_lists and run_layers (epnn_api.cu), FP32, one
+// chunk.  The only code that is not the product's is this orchestration (without streams and workspaces), the host-side
+// scans and the row groups of the large systems (sys_prep_kernel, rg_fill_kernel).
 // tests/test_emu_infer.py compares the result with the oracle and with the reference's shipped predictions.
 // Build: g++ -O1 -std=c++17 -ffp-contract=off -shared -fPIC -pthread -DEPNN_CPU_EMU -o build/libemu_infer.so tools/emu/emu_infer.cpp
 #define EPNN_CPU_EMU 1
@@ -48,8 +48,17 @@ static void exclusive_scan(const int* in, int* out, int n) { int s = 0; for (int
 extern "C" int emu_infer(int T, int n_x, const float* w_packed, size_t n_w, int n_sys, const int* off, const float* xyz,
                          const int* species, const float* Q, const int* npad_in, int variant, int dedup,
                          float* q_out, double* q_out64, float* h_out, long long* dedup_rows_out) {
-    if (n_w != expected_floats(T, n_x)) return -1;
-    const int pair_const = variant == 1, pair_tensor = variant == 2, run_set = variant == 3;
+    if (n_w != expected_floats(T, n_x) || variant < 0 || variant > 3) return -1;
+    // variant: 0 "pair_const" 0, 1 "pair_const" 1, 2 "pair_const" 0 with "pair_tensor" 1, 3 "pair_const" 2 (the shipped set)
+    KernelOptions opt;
+    opt.pair_const = variant == 1 ? 1 : variant == 3 ? 2 : 0;
+    opt.pair_tensor = variant == 2;
+    opt.far_tensor = 0;
+    const KernelChoice kc = resolve_kernels(32, 0, opt);
+    // one SM: the partial-sum planes grow with the SM count; at one the 49..90-atom systems of the tests still get 3 to 16
+    constexpr int kSmCount = 1;
+    ChunkPlan pl;
+    if (!plan_chunk(off, n_sys, kSmCount, 0, 1, kc, pl)) return -1;
     const int n = off[n_sys];
     const int n_species = n_x - 1;
     // ---------------------------------------------------------------- weights: the product's own packing and folding
@@ -72,17 +81,12 @@ extern "C" int emu_infer(int T, int n_x, const float* w_packed, size_t n_w, int 
     for (int s = 0; s < n_sys; ++s) npad[s] = npad_in ? npad_in[s] : off[s + 1] - off[s];
     std::vector<double> q(n);
     emu_launch_simple(div_up(n, 256), 256, [&] { k_nbr::prep_kernel(n, n_sys, off, Q, atom_sys.data(), q.data()); });
-    std::vector<int> large, lbase;
-    long long cells = 0;
-    for (int s = 0; s < n_sys; ++s) {
-        const int ns = off[s + 1] - off[s];
-        if (ns > CELL_MIN) { large.push_back(s); lbase.push_back((int)cells); cells += 4ll * ns + 64; }
-    }
+    const long long cells = pl.n_cells;
     std::vector<CellGrid> grid(n_sys + 1);
     std::vector<int> cell_start((size_t)cells + 2, 0), cell_atoms(n + 1, 0);
-    if (!large.empty()) {
+    if (pl.n_large) {
         std::vector<int> cnt((size_t)cells + 2, 0);
-        emu_launch_grid((int)large.size(), 8, 0, [&] { k_nbr::cell_setup_kernel((int)large.size(), large.data(), lbase.data(), off, xyz, grid.data()); });
+        emu_launch_grid(pl.n_large, 8, 0, [&] { k_nbr::cell_setup_kernel(pl.n_large, pl.cell_tab.data(), pl.cell_tab.data() + pl.n_large, off, xyz, grid.data()); });
         emu_launch_simple(div_up(n, 256), 256, [&] { k_nbr::cell_bin_kernel<0>(n, atom_sys.data(), off, xyz, grid.data(), cnt.data(), nullptr, nullptr); });
         exclusive_scan(cnt.data(), cell_start.data(), (int)cells);
         std::fill(cnt.begin(), cnt.end(), 0);
@@ -106,18 +110,7 @@ extern "C" int emu_infer(int T, int n_x, const float* w_packed, size_t n_w, int 
         emu_launch_grid(div_up(Pn, EDGE_PAIRS), EDGE_PAIRS / 32, 0, [&] { k_nbr::edge_desc_kernel<EDR>((int64_t)Pn, pair_D.data(), e.data(), near.data(), nullptr, nullptr, nullptr, nullptr); });
 
     // ---------------------------------------------------------------- bundles, far lists, row groups, species tables
-    std::vector<int2> bundles;
-    {
-        int cur0 = -1, cur_n = 0;
-        for (int s = 0; s < n_sys; ++s) {
-            const int a0 = off[s], ns = off[s + 1] - off[s];
-            if (ns > SMALL_MAX) { if (cur_n) { bundles.push_back(make_int2(cur0, cur_n)); cur_n = 0; } continue; }
-            if (cur_n && cur_n + ns > BUNDLE_ATOMS) { bundles.push_back(make_int2(cur0, cur_n)); cur_n = 0; }
-            if (!cur_n) cur0 = a0;
-            cur_n += ns;
-        }
-        if (cur_n) bundles.push_back(make_int2(cur0, cur_n));
-    }
+    std::vector<int2> bundles = pl.bundles;
     const int n_bundles = (int)bundles.size();
     bundles.push_back(make_int2(0, 0));
     std::vector<int> far_cnt(n + 1, 0), far_off(n + 1, 0), far0_cnt(n + 1, 0), far0_off(n + 1, 0), rep(n + 1, 0), atom_b0(n + 1, 0), bundle_nat(n + 1, 0);
@@ -127,7 +120,7 @@ extern "C" int emu_infer(int T, int n_x, const float* w_packed, size_t n_w, int 
     std::vector<unsigned short> far_list(far_off[n] + 2), far0_list((size_t)(MAX_SPECIES + 1) * n + 2);
     std::vector<unsigned char> far0_w((size_t)(MAX_SPECIES + 1) * n + 16);
     if (n_bundles) {
-        if (Pn > 0)
+        if (kc.tile_perm && Pn > 0)
             emu_launch_simple(div_up(Pn, 256), 256, [&] {
                 k_bundle::tile_perm_kernel((int64_t)Pn, pair_i.data(), pair_j.data(), atom_sys.data(), off, atom_b0.data(), ustart.data(),
                                            bundle_nat.data(), perm_j.data()); });
@@ -143,7 +136,7 @@ extern "C" int emu_infer(int T, int n_x, const float* w_packed, size_t n_w, int 
             k_bundle::far0_kernel<1>(n, atom_sys.data(), off, npad.data(), species, rowptr.data(), col.data(), atom_b0.data(), nullptr, nullptr,
                                      far0_off.data(), far0_list.data(), far0_w.data()); });
     std::vector<unsigned char> rowl(nnz + 16, 0);
-    if (run_set && n_bundles && nnz > 0)
+    if (kc.csr_rowl && n_bundles && nnz > 0)
         emu_launch_simple(div_up(n, 256), 256, [&] { k_brun::csr_rowl_kernel(n, atom_sys.data(), off, rowptr.data(), atom_b0.data(), rowl.data()); });
     std::vector<int> rgl_off(n_sys + 1, 0), rg;
     for (int s = 0; s < n_sys; ++s) {
@@ -151,9 +144,9 @@ extern "C" int emu_infer(int T, int n_x, const float* w_packed, size_t n_w, int 
         rgl_off[s + 1] = rgl_off[s] + (ns > SMALL_MAX ? (ns + 3) >> 2 : 0);
         if (ns > SMALL_MAX) for (int i = off[s]; i < off[s + 1]; i += 4) rg.push_back(i);
     }
-    const int n_rg = (int)rg.size();
+    const int n_rg = pl.n_rg_large;
     rg.push_back(0);
-    const int nsplit = n_rg > 0 ? 3 : 1;                 // a few partial-sum planes, to exercise their fixed-order addition
+    const int nsplit = pl.nsplit;
     const int n_sp_tab = n_rg / 8 + 2;
     std::vector<int> sp_tab((size_t)n_sp_tab * 32, 0), sp_stamp((size_t)n_sp_tab * 2, 0);
     unsigned long long dedup_rows = 0;
@@ -170,7 +163,7 @@ extern "C" int emu_infer(int T, int n_x, const float* w_packed, size_t n_w, int 
     constexpr int NW = 8;
 
     auto atom = [&](int mode, const StepW<float>* prev, const StepW<float>* next, int h_is_zero) {
-        if (pair_const) {
+        if (kc.atom == ATOM_K_CONST) {
             k_aconst::AtomW W;
             memset(&W, 0, sizeof(W));
             k_aconst::AtomConstArgs aa;
@@ -204,7 +197,7 @@ extern "C" int emu_infer(int T, int n_x, const float* w_packed, size_t n_w, int 
     auto bundle = [&](bool epn, const StepW<float>& sw) {
         if (!n_bundles) return;
         work_counter = 0;
-        if (pair_tensor && epn) {
+        if (epn && kc.epn == EPN_MMA) {
             k_mma::EpnMmaArgs a;
             a.n_bundles = n_bundles; a.bundle = bundles.data(); a.work_counter = &work_counter;
             a.ustart = ustart.data(); a.pair_i = pair_i.data(); a.pair_j = pair_j.data(); a.near = near.data(); a.e = e.data();
@@ -212,7 +205,7 @@ extern "C" int emu_infer(int T, int n_x, const float* w_packed, size_t n_w, int 
             emu_launch_cta(MMA_NW, (size_t)MMA_NW * BUNDLE_ATOMS * UVS, [&] { k_mma::bundle_epn_mma_kernel(a); });
             return;
         }
-        if (run_set && !epn) {
+        if (!epn && kc.gnn == GNN_RUN) {
             k_brun::RunW W;
             memcpy(W.W2, sw.W2, sizeof(W.W2));
             k_brun::RunArgs a;
@@ -226,7 +219,7 @@ extern "C" int emu_infer(int T, int n_x, const float* w_packed, size_t n_w, int 
             emu_launch_cta(RUN_NW, k_brun::RunSmem::bytes() / sizeof(float), [&] { k_brun::bundle_run_kernel(W, &a); });
             return;
         }
-        if (pair_const || run_set) {
+        if (epn ? kc.epn == EPN_CONST : kc.gnn == GNN_CONST) {
             k_bconst::PairW W;
             memcpy(W.W2, sw.W2, sizeof(W.W2));
             k_bconst::ConstArgs a;
@@ -251,7 +244,7 @@ extern "C" int emu_infer(int T, int n_x, const float* w_packed, size_t n_w, int 
         else     emu_launch_cta(NW, k_bundle::BundleSmem<float, false>::bytes(NW) / sizeof(float) + 8, [&] { k_bundle::bundle_kernel<float, NW, false>(a); });
     };
 
-    // ---------------------------------------------------------------- GNN layer (charge_gn.py:60-74), launch order of run_chunk
+    // ---------------------------------------------------------------- GNN layer (charge_gn.py:60-74), launch order of run_layers
     atom(ATOM_PROJECT, nullptr, &msg[0], 1);
     for (int t = 0; t < T; ++t) {
         bundle(false, msg[t]);
@@ -262,23 +255,22 @@ extern "C" int emu_infer(int T, int n_x, const float* w_packed, size_t n_w, int 
                     k_gnn::sp_check_kernel<float>(n, atom_sys.data(), off, species, rgl_off.data(), sp_tab.data(), v.data(), sp_stamp.data(), stamp); });
                 emu_launch_simple(div_up(n_sp_tab, 256), 256, [&] { k_gnn::sp_tally_kernel(n_sp_tab, sp_tab.data(), sp_stamp.data(), stamp, &dedup_rows); });
             }
-            // variants 1 and 3: the far columns of the live steps go to the row-per-thread kernel (planes 0 .. nsplit - 2), gnn_pair_kernel
-            // keeps the near pairs, the pad pair and the species slots on the last plane -- the far_tc == 2 arrangement of run_chunk
-            const bool far_const = pair_const || run_set;
+            // FAR_CONST: the far columns of the live steps go to the row-per-thread kernel (planes 0 .. nsplit - 2), gnn_pair_kernel
+            // keeps the near pairs, the pad pair and the species slots on the last plane
+            const bool far_const = pl.far == FAR_CONST;
             if (far_const) {
-                std::vector<int2> blk;
-                for (int s = 0; s < n_sys; ++s)
-                    if (off[s + 1] - off[s] > SMALL_MAX) for (int i = off[s]; i < off[s + 1]; i += 32) blk.push_back(make_int2(i, s));
                 k_farc::FarW FW;
                 memcpy(FW.W2, msg[t].W2, sizeof(FW.W2)); memcpy(FW.b2, msg[t].b2, sizeof(FW.b2));
                 k_farc::FarConstArgs fa;
-                fa.blk = blk.data(); fa.nsplit = nsplit - 1; fa.n_atoms = n; fa.unit_begin = 0; fa.unit_end = (int)blk.size() * (nsplit - 1);
+                fa.blk = pl.rowblk.data(); fa.nsplit = nsplit - 1; fa.n_atoms = n;
+                fa.unit_begin = pl.blk_begin * (nsplit - 1); fa.unit_end = pl.blk_end * (nsplit - 1);
                 fa.sys_off = off; fa.rowptr = rowptr.data(); fa.col = col.data(); fa.u = u.data(); fa.v = v.data(); fa.S = S.data();
                 fa.rgl_off = rgl_off.data(); fa.sp_stamp = sp_stamp.data(); fa.stamp = stamp;
                 emu_launch_grid(2, FARC_NW, (size_t)FARC_NW * FARC_PW_BYTES / sizeof(float) + 8, [&] { k_farc::gnn_far_const_kernel(FW, fa); });
             }
             k_gnn::GnnArgs<float> ga;
-            ga.rg_atom = rg.data(); ga.unit_begin = 0; ga.n_units = far_const ? n_rg : n_rg * nsplit; ga.nsplit = far_const ? 1 : nsplit; ga.n_atoms = n;
+            const int ns = far_const ? 1 : nsplit;
+            ga.rg_atom = rg.data(); ga.unit_begin = pl.rg_begin * ns; ga.n_units = pl.rg_end * ns; ga.nsplit = ns; ga.n_atoms = n;
             ga.skip_far = far_const ? 1 : 0; ga.plane = far_const ? nsplit - 1 : 0;
             ga.atom_sys = atom_sys.data(); ga.sys_off = off; ga.npad = npad.data(); ga.rowptr = rowptr.data(); ga.col = col.data(); ga.pid = pid.data();
             ga.e = e.data(); ga.u = u.data(); ga.v = v.data(); ga.Cw = msg[t].Cw; ga.W2 = msg[t].W2; ga.b2 = msg[t].b2; ga.b1 = msg[t].b1; ga.S = S.data();

@@ -1,6 +1,6 @@
 // CPU emulation driver for the neighbour-list and descriptor kernels, epnn_b200/csrc/epnn_neighbor.cu (test
-// infrastructure; see cuda_emu.h).  Same launch sequence as run_chunk (epnn_api.cu): prep -> cell build (systems with
-// more than `cell_min_override` atoms... the kernels' own CELL_MIN) -> count -> scans -> fill -> reverse edges -> descriptors.
+// infrastructure; see cuda_emu.h).  Same launch sequence as build_lists (epnn_api.cu): prep -> cell build (systems with
+// more than CELL_MIN atoms, cell bases of plan_cells, epnn_plan.h) -> count -> scans -> fill -> reverse edges -> descriptors.
 // Build: g++ -O1 -std=c++17 -ffp-contract=off -shared -fPIC -pthread -DEPNN_CPU_EMU -o build/libemu_neighbor.so tools/emu/emu_neighbor.cpp
 #define EPNN_CPU_EMU 1
 #include "../../epnn_b200/csrc/epnn_neighbor.cu"
@@ -12,18 +12,14 @@ extern "C" int emu_neighbor_counts(const double* mu, const double* B, int n_atom
                                    int* grid_ints /* 8 ints per system */, int* cell_start, int* cell_atoms, int n_cells_cap) {
     emu_set_rbf(mu, B);
     emu_launch_simple(div_up(n_atoms, 256), 256, [&] { prep_kernel(n_atoms, n_sys, sys_off, Qsys, atom_sys, q0); });
-    // cell lists of the big systems: host-side budget of 4 n + 64 cells each, as in run_chunk
-    std::vector<int> large, base;
-    long long cells = 0;
-    for (int s = 0; s < n_sys; ++s) {
-        const int n = sys_off[s + 1] - sys_off[s];
-        if (n > CELL_MIN) { large.push_back(s); base.push_back((int)cells); cells += 4ll * n + 64; }
-    }
+    std::vector<int> tab;
+    const long long cells = plan_cells(sys_off, n_sys, tab);
+    const int n_large = (int)tab.size() / 2;
     if (cells + 1 > n_cells_cap) return -1;
     CellGrid* grid = reinterpret_cast<CellGrid*>(grid_ints);
-    if (!large.empty()) {
+    if (n_large) {
         std::vector<int> cnt((size_t)cells + 2, 0);
-        emu_launch_grid((int)large.size(), 8, 0, [&] { cell_setup_kernel((int)large.size(), large.data(), base.data(), sys_off, xyz, grid); });
+        emu_launch_grid(n_large, 8, 0, [&] { cell_setup_kernel(n_large, tab.data(), tab.data() + n_large, sys_off, xyz, grid); });
         emu_launch_simple(div_up(n_atoms, 256), 256, [&] { cell_bin_kernel<0>(n_atoms, atom_sys, sys_off, xyz, grid, cnt.data(), nullptr, nullptr); });
         exclusive_scan(cnt.data(), cell_start, (int)cells);
         std::fill(cnt.begin(), cnt.end(), 0);
